@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- exact kNN queries/sec on the BASELINE.json headline workload, plus BASELINE configs 1-5.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--configs all|none|c1,c3,...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--configs all|none|c1,c3,...] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Headline workload (BASELINE.json metric): 10M x 768 fp32 rows, cosine, k=10, batch-1 queries; with N GPUs the rows are
@@ -32,6 +32,11 @@ One JSON line on rank 0:
 
 ``--impl reference`` times that CPU implementation as the reference arm (the reference's own search is the absent
 hnswlib wheel; see DESIGN.md) with every host core it may use and prints the same line with impl=reference.
+
+``--dump-outputs DIR`` writes what the device path returned for the queries of the last timed headline step:
+distances.npy [nq, k] float32, rows.npy [nq, k] and counts.npy [nq] as float64, and query_index.npy (which queries of the
+step they are; all of them unless the step's results exceed 60 MB).  Rows and queries come from fixed seeds, so two runs
+with the same arguments see the same inputs.
 """
 from __future__ import annotations
 
@@ -58,7 +63,8 @@ PART_SHIFT = 40
 def parse_args():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=10)
+    ap.add_argument("--steps", type=int, default=10,
+                    help="timed steps of the headline region and of its e2e measurement (configs c1-c5 time fixed repetitions)")
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", type=int, default=10_000_000)
@@ -76,7 +82,15 @@ def parse_args():
     ap.add_argument("--parity-queries", type=int, default=4, help="timed queries checked against the streamed oracle (0 = skip)")
     ap.add_argument("--configs", default="all", help="all | none | comma list of c1,c2,c3,c4,c5")
     ap.add_argument("--configs-scale", type=float, default=1.0, help="scale the configs' row counts (development runs)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed headline step to DIR/<name>.npy (float32/float64) so that "
+                         "two builds can be compared output for output")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl == "reference":
+        ap.error("--dump-outputs writes the device path's results; the reference arm has none to write")
+    return a
 
 
 def workload_config(a, n_gpus):
@@ -92,6 +106,24 @@ def workload_config(a, n_gpus):
 
 def make_queries(nq, dim):
     return np.random.default_rng(SEED + 1).standard_normal((nq, dim), dtype=np.float32)
+
+
+DUMP_MAX_BYTES = 60_000_000      # data; the four .npy headers add 512 bytes, the whole dump stays under 64 MB
+
+
+def dump_outputs(out_dir, dists, rows, counts):
+    """Write one step's results (dists [nq, k] fp32, global rows [nq, k], counts [nq]) as .npy files.  Ids go out as
+    float64 (exact below 2**53).  Past DUMP_MAX_BYTES a fixed seeded sample of the queries is written;
+    query_index.npy says which."""
+    nq, k = dists.shape
+    per_query = k * (4 + 8) + 8 + 8
+    keep = np.arange(nq)
+    if nq * per_query > DUMP_MAX_BYTES:
+        keep = np.sort(np.random.default_rng(SEED).choice(nq, DUMP_MAX_BYTES // per_query, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, arr in (("distances", dists[keep].astype(np.float32)), ("rows", rows[keep].astype(np.float64)),
+                      ("counts", counts[keep].astype(np.float64)), ("query_index", keep.astype(np.float64))):
+        np.save(os.path.join(out_dir, f"{name}.npy"), arr)
 
 
 def hbm_peak():
@@ -309,8 +341,10 @@ def run_ours(a):
     k = a.k
     inflight = max(1, min(a.inflight, 2))
     streams = [torch.cuda.Stream(device) for _ in range(inflight)]
+    # one result buffer per query of a step, so that the whole last step is still there when it is read back
     outs = [(torch.empty((1, k), dtype=torch.float32, device=device), torch.empty((1, k), dtype=torch.int64, device=device),
-             torch.empty((1,), dtype=torch.int32, device=device)) for _ in range(inflight)]
+             torch.empty((1,), dtype=torch.int32, device=device)) for _ in range(qps_step)]
+    step_results = [None] * qps_step
 
     def device_query(j, st, o):
         """ONE batch-1 search through the C ABI with device pointers, on stream st, results into o."""
@@ -325,7 +359,7 @@ def run_ours(a):
         # every query is its own search (own launch, own result); `lanes` of them are in flight, each
         # on its own stream, so one query's scan fills the SMs the previous one's tail has left
         for j in range(qps_step):
-            device_query(j, streams[j % lanes], outs[j % lanes])
+            step_results[j] = device_query(j, streams[j % lanes], outs[j])
 
     def api_search(j):
         return index.search(VectorDTO(values=Q[j], metadata={}), top_k=k, namespace=ns, metric=a.space)
@@ -358,6 +392,8 @@ def run_ours(a):
     sampler.start()
     ms_total = ctx.timed(step_device, a.steps, streams)
     sampler.stop()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, *(torch.cat([r[i] for r in step_results]).cpu().numpy() for i in range(3)))
     half1 = shard.gemm_stats()
     half_q = half1["half_scan_queries"] - half0["half_scan_queries"]           # searches that read the fp16 shadow
     half_u = half1["half_scan_uncertified"] - half0["half_scan_uncertified"]   # ... re-run by the fp32 launch behind

@@ -1,22 +1,25 @@
 """Import the UNMODIFIED reference wrappers over the exact hnswlib stand-in.  TEST ORACLE.
 
-Only usable where ``/root/reference`` exists (this build container, never the GPU box).
+Needs a checkout of the original MLVectorDB project at ``BASELINE.json``'s ``reference_path``
+(``MLV_REFERENCE_ROOT`` overrides it).
 The reference modules import each other as ``src.mlvectordb...`` and need the reference
 root on ``sys.path`` (reference ``storage_engine_in_memory.py:6-7``, ``pyproject.toml:6``);
 ``src/mlvectordb/__init__.py:19`` imports ``Index`` eagerly, which imports ``hnswlib`` --
 so ``sys.modules['hnswlib']`` is pre-seeded with ``oracle.hnswlib_exact``.
 
-Used by ``tests/golden/make_golden.py`` to generate the committed fixtures and by the
-CPU-side tests that re-run the reference's own test-suite against the stand-in.
+Used by ``tests/golden/make_golden.py`` to generate the committed fixtures, which the tests replay
+without the reference.
 """
 from __future__ import annotations
 
 import importlib
+import json
 import os
 import sys
 from types import SimpleNamespace
 
-REFERENCE_ROOT = os.environ.get("MLV_REFERENCE_ROOT", "/root/reference")
+with open(os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "BASELINE.json")) as _f:
+    REFERENCE_ROOT = os.environ.get("MLV_REFERENCE_ROOT", json.load(_f)["reference_path"])
 
 
 def available() -> bool:

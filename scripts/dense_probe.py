@@ -1,5 +1,5 @@
 import json, os, sys
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 from mlvectordb_b200 import DeviceShard
 from oracle import synthetic
 dim, nq, k = 768, 4096, 100

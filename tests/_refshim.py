@@ -1,13 +1,12 @@
 """Test-only stand-ins for the reference's CALLERS of the index (not part of the product).
 
-``/root/reference`` does not exist on the GPU box, so the drop-in tests need a thin
+The original project is not part of this repository, so the drop-in tests need a thin
 restatement of what sits around the index: ``Vector`` (reference
 ``src/mlvectordb/implementations/vector.py:10-42``), an in-memory storage
 (``storage_engine_in_memory.py:10-86``, only the calls ``QueryProcessor`` makes) and
 ``QueryProcessor`` (``query_processor.py:11-62``).  Behaviour restated, not copied: uuid4 ids,
 fp32 value copies, hit enrichment in hit order dropping ids missing from storage, delete ->
-remove -> rebuild-if-flagged.  Where the reference tree is present the CPU tests also run the
-real classes (``oracle/refload.py``).
+remove -> rebuild-if-flagged.
 """
 from __future__ import annotations
 

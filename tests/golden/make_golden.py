@@ -1,9 +1,9 @@
 """Generate ``tests/golden/reference_wrappers.json``.
 
-Runs the UNMODIFIED reference ``Index`` / ``QueryProcessor`` (imported from /root/reference,
-reference ``src/mlvectordb/implementations/index.py`` and ``query_processor.py``) over the
-exact hnswlib stand-in (``oracle/hnswlib_exact.py``) and records what they return.  The
-reference cannot travel to the GPU box, so the outputs are committed; the inputs are
+Runs the UNMODIFIED reference ``Index`` / ``QueryProcessor`` (imported from the original project's
+checkout at ``BASELINE.json``'s ``reference_path`` or ``MLV_REFERENCE_ROOT``, reference
+``src/mlvectordb/implementations/index.py`` and ``query_processor.py``) over the exact hnswlib stand-in (``oracle/hnswlib_exact.py``) and records what
+they return.  The reference is not part of this repository, so the outputs are committed; the inputs are
 regenerated from ``oracle/synthetic.py`` by the tests (only seeds are stored).
 
 PARITY UNPINNED: the arithmetic under the wrappers is the oracle's restatement of hnswlib
@@ -11,7 +11,7 @@ PARITY UNPINNED: the arithmetic under the wrappers is the oracle's restatement o
 behaviour (clamping, score transform, tombstones, rebuild, ordering), and the oracle's
 numbers at the time of generation.
 
-Usage (in the build container):  python tests/golden/make_golden.py
+Usage:  python tests/golden/make_golden.py
 """
 from __future__ import annotations
 

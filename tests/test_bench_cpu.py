@@ -34,6 +34,37 @@ def test_reference_arm_uses_every_core_under_torchrun_env():
     assert line["cpu_baseline"]["row_prefix_used"] is False and line["config"]["queries_per_step"] == 4
 
 
+def test_steps_below_one_and_dump_of_reference_arm_are_refused(tmp_path):
+    for args, flag in ((["--steps", "0"], "--steps"), (["--dump-outputs", str(tmp_path / "d")], "--dump-outputs")):
+        out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", *args],
+                             capture_output=True, text=True, timeout=60, cwd=ROOT)
+        assert out.returncode == 2 and flag in out.stderr
+    assert not (tmp_path / "d").exists()
+
+
+def test_dump_outputs_files_and_size_cap(tmp_path, monkeypatch):
+    import numpy as np
+    import bench
+    rng = np.random.default_rng(0)
+    nq, k = 40, 10
+    d = rng.random((nq, k), dtype=np.float32)
+    r = rng.integers(0, 1 << 45, (nq, k))
+    c = np.full(nq, k, np.int32)
+    bench.dump_outputs(str(tmp_path / "all"), d, r, c)
+    got = {n: np.load(tmp_path / "all" / f"{n}.npy") for n in ("distances", "rows", "counts", "query_index")}
+    assert got["distances"].dtype == np.float32 and np.array_equal(got["distances"], d)
+    assert got["rows"].dtype == np.float64 and np.array_equal(got["rows"].astype(np.int64), r)
+    assert np.array_equal(got["counts"], c) and np.array_equal(got["query_index"], np.arange(nq))
+    # past the cap: the same fixed sample of queries every time, and the files stay under it
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 10 * (k * 12 + 16))
+    for sub in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / sub), d, r, c)
+    idx = np.load(tmp_path / "a" / "query_index.npy")
+    assert len(idx) == 10 and np.array_equal(idx, np.load(tmp_path / "b" / "query_index.npy"))
+    assert np.array_equal(np.load(tmp_path / "a" / "distances.npy"), d[idx.astype(np.int64)])
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= 10 * (k * 12 + 16) + 4 * 128   # + .npy headers
+
+
 def test_reference_arm_other_ranks_exit_quietly():
     env = dict(os.environ, RANK="1", WORLD_SIZE="2")
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2"],
