@@ -421,6 +421,23 @@ int mlv_index_gemm_stats(mlv_index_t h, mlv_gemm_stats_t *out);
  * NaN for tombstoned rows.  1 <= rows <= 8192, dim >= 32.
  */
 int mlv_index_debug_gemm(mlv_index_t h, const float *queries, uint32_t nq, float *out_approx);
+/*
+ * Debug / bound tests: the APPROXIMATE distances the shadow scan's consumers compute for ONE host query against every
+ * stored row (the same consumer code: FMA or tensor-core consumers, whichever "scan_half_mma" and the row length select
+ * for a search), before any re-scoring: out_approx[rows], +inf for tombstoned rows.  *out_info receives what the
+ * certificate and the range margin are computed from.  1 <= rows <= 8192.
+ */
+typedef struct mlv_half_scan_debug {
+    float delta_rel;    /* bound on |approx - exact| / scale (gemm_kernel.cuh, gemm_delta_rel_f16) */
+    float scale;        /* as the kernel computed it: (sqrt(max_norm2) + |q|)^2 for l2, sqrt(max_norm2) |q| for ip, 1 for cosine */
+    float q_norm2;      /* |q|^2 of the prepared query, as the kernel computed it */
+    float max_norm2;    /* largest |x|^2 of the rows (0 for cosine: unit rows) */
+    float x_unscale;    /* 2^-s: the shadow holds halves of row * 2^s, s frozen when the shadow was built */
+    float q_unscale;    /* 2^-t: the tensor-core consumers multiply halves of q * 2^t (1 for the FMA consumers) */
+    uint32_t overflow;  /* rows appended after the scale froze overflowed fp16: searches do not trust the shadow */
+    uint32_t consumers; /* 1 = FMA consumers, 2 = tensor-core consumers (mma.sync) */
+} mlv_half_scan_debug_t;
+int mlv_index_debug_half_scan(mlv_index_t h, const float *query, float *out_approx, mlv_half_scan_debug_t *out_info);
 /* Kernels launched by this handle since creation (scan + select + maintenance). */
 int mlv_index_kernel_launches(mlv_index_t h, uint64_t *launches);
 

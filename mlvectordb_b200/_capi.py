@@ -51,6 +51,20 @@ class GemmStats(C.Structure):
     ]
 
 
+class HalfScanDebug(C.Structure):
+    """``mlv_half_scan_debug_t``"""
+    _fields_ = [
+        ("delta_rel", C.c_float),
+        ("scale", C.c_float),
+        ("q_norm2", C.c_float),
+        ("max_norm2", C.c_float),
+        ("x_unscale", C.c_float),
+        ("q_unscale", C.c_float),
+        ("overflow", C.c_uint32),
+        ("consumers", C.c_uint32),
+    ]
+
+
 class Predicate(C.Structure):
     """``mlv_predicate_t``"""
     _fields_ = [("column", C.c_uint32), ("op", C.c_int32), ("a", C.c_int32), ("b", C.c_int32)]
@@ -131,6 +145,7 @@ SIGNATURES = {
     "mlv_index_collect": (C.c_int, [_h, C.c_uint32, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mlv_index_gemm_stats": (C.c_int, [_h, C.POINTER(GemmStats)]),
     "mlv_index_debug_gemm": (C.c_int, [_h, C.c_void_p, C.c_uint32, C.c_void_p]),
+    "mlv_index_debug_half_scan": (C.c_int, [_h, C.c_void_p, C.c_void_p, C.POINTER(HalfScanDebug)]),
 }
 
 _lib = None

@@ -1401,6 +1401,64 @@ int mlv_index_debug_gemm(mlv_index_t h, const float* queries, uint32_t nq, float
     return MLV_OK;
 }
 
+int mlv_index_debug_half_scan(mlv_index_t h, const float* query, float* out_approx, mlv_half_scan_debug_t* out_info) {
+    if (!h) return MLV_E_INVALID;
+    if (!query || !out_approx || !out_info) return fail(h, MLV_E_INVALID, "bad argument");
+    if (h->rows == 0 || h->rows > SELECT_MAX_P || h->ld < 8) return fail(h, MLV_E_UNSUPPORTED, "debug_half_scan needs 1..8192 rows and dim >= 8");
+    DeviceGuard g(h->device);
+    cudaStream_t st = h->stream;
+    Lane* ln = lane_for(h, st);
+    int rc;
+    if ((rc = ensure_dev(h, h->d_qraw, (size_t)h->dim * 4)) != MLV_OK) return rc;
+    CK(h, cudaMemcpyAsync(h->d_qraw.p, query, (size_t)h->dim * 4, cudaMemcpyHostToDevice, st));
+    if ((rc = prep_queries(h, (const float*)h->d_qraw.p, 1, st)) != MLV_OK) return rc;
+    if (h->metric != MLV_COSINE && (rc = ensure_row_norms(h, st)) != MLV_OK) return rc;
+    bool usable = false;
+    if ((rc = ensure_f16_shadow(h, st, &usable)) != MLV_OK) return rc;
+    if (!usable) return fail(h, MLV_E_NOMEM, "no room for the fp16 shadow");
+    const int half_kind = (f16_ld(h) % 64 == 0 && h->tune_scan_half_mma != 0) ? 2 : 1;   // search_prepared's choice
+    ScanCfg c;
+    if ((rc = choose_cfg(h, 1, 1, true, &c, false, half_kind)) != MLV_OK) return rc;
+    ScanParams p = scan_params(h, c, FilterPlan{}, ln, 1);
+    p.sched = nullptr;
+    p.rows = reinterpret_cast<const float4*>(h->d_rows16.p);
+    p.ld4 = f16_ld(h) / 8;
+    p.rows_exact = reinterpret_cast<const float4*>(h->d_rows);
+    p.ld4_exact = h->ld / 4;
+    p.half_state = (const uint32_t*)h->d_f16st.p;
+    p.row_norms = h->metric == MLV_L2 ? (const float*)h->d_norms.p : nullptr;
+    p.max_norm2_bits = h->metric == MLV_COSINE ? nullptr : (const uint32_t*)h->d_maxn2.p;
+    p.delta_rel = gemm_delta_rel_f16_host(h->metric == MLV_L2, h->ld);
+    p.cosine = h->metric == MLV_COSINE;
+    p.queries = reinterpret_cast<const float4*>(ln->d_q.p);
+    p.nq_valid = 1;
+    // [rows] approximate distances (+inf where the kernel stores nothing) | |q|^2, 2^-s 2^-t, scale
+    const size_t n_out = (size_t)h->rows + 3;
+    if ((rc = ensure_dev(h, h->d_outd, n_out * 4)) != MLV_OK) return rc;
+    std::vector<float> out(n_out, std::numeric_limits<float>::infinity());
+    CK(h, cudaMemcpyAsync(h->d_outd.p, out.data(), n_out * 4, cudaMemcpyHostToDevice, st));
+    p.out_dists = (float*)h->d_outd.p;
+    CK(h, h->metric == MLV_L2 ? launch_scan_half_debug_m<METRIC_L2>(p, c, st) : launch_scan_half_debug_m<METRIC_IP>(p, c, st));
+    h->launches++;
+    uint32_t f16st[3] = {0, 0, 0}, maxn2 = 0;
+    CK(h, cudaMemcpyAsync(out.data(), h->d_outd.p, n_out * 4, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(f16st, h->d_f16st.p, 12, cudaMemcpyDeviceToHost, st));
+    if (h->metric != MLV_COSINE) CK(h, cudaMemcpyAsync(&maxn2, h->d_maxn2.p, 4, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaStreamSynchronize(st));
+    memcpy(out_approx, out.data(), (size_t)h->rows * 4);
+    float x_unscale;
+    memcpy(&x_unscale, &f16st[0], 4);
+    memcpy(&out_info->max_norm2, &maxn2, 4);
+    out_info->delta_rel = p.delta_rel;
+    out_info->q_norm2 = out[h->rows];
+    out_info->x_unscale = x_unscale;
+    out_info->q_unscale = out[h->rows + 1] / x_unscale;   // powers of two: exact
+    out_info->scale = out[h->rows + 2];
+    out_info->overflow = f16st[2];
+    out_info->consumers = c.R == 16 ? 2u : 1u;   // rows too long for two 16-row stages take the FMA consumers
+    return MLV_OK;
+}
+
 int mlv_index_debug_timeline(mlv_index_t h, uint64_t* out, uint32_t max_ctas, uint32_t* n_ctas) {
     if (!h || !out || !n_ctas) return MLV_E_INVALID;
     DeviceGuard g(h->device);

@@ -269,13 +269,17 @@ __device__ __forceinline__ void mma_m16n8k16_f16(float (&c)[4], uint32_t a0, uin
                  : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
-template <int METRIC, int NQ, int R, bool RANGE, bool INLINE, int HALF = 0>
+template <int METRIC, int NQ, int R, bool RANGE, bool INLINE, int HALF = 0, bool DEBUG = false>
 __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) {
     constexpr int V = R * NQ;
     static_assert(V <= 32 && (V & (V - 1)) == 0, "R*NQ must be a power of two <= 32");
     // HALF: 0 = the fp32 rows; 1 = the fp16 shadow, FMA consumers; 2 = the fp16 shadow, tensor-core consumers
     // (mma.sync m16n8k16 on 16 rows x 64 halves per step, the query as halves too; rows of a multiple of 64 halves)
     static_assert(!HALF || (NQ == 1 && !INLINE), "the shadow scan takes one prepared query");
+    // DEBUG (scan_kernel_half_debug): the shadow range instantiation's set-up and consumers, but every live row's
+    // approximate distance is stored to out_dists[row] instead of being tested, then {|q|^2, 2^-s 2^-t, scale} to
+    // out_dists[n_rows ..]; static tile schedule (sched == nullptr), no tail
+    static_assert(!DEBUG || (HALF && RANGE), "the debug view is of the shadow range scan");
     static_assert(HALF != 2 || R == 16, "the tensor-core consumers score 16 rows per step");
     constexpr bool HMMA = HALF == 2;
     extern __shared__ __align__(128) unsigned char smem[];
@@ -390,6 +394,11 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
             const bool over = __ldg(p.half_state + 2) != 0;
             half_margin = over ? __int_as_float(0x7f800000) : p.delta_rel * scale;
             if (over && p.half_stats_host && blockIdx.x == 0 && tid == 0) p.half_stats_host[2] = 1;
+            if (DEBUG && blockIdx.x == 0 && tid == 0) {
+                p.out_dists[p.n_rows] = half_qn;
+                p.out_dists[p.n_rows + 1] = half_us;
+                p.out_dists[p.n_rows + 2] = scale;
+            }
         }
     } else {
         // queries -> shared (missing queries of a short group repeat the last one; masked later)
@@ -628,7 +637,9 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
                 dist = (METRIC == METRIC_IP) ? 1.0f - s : s;
             const uint64_t key = make_key(dist, row);
             const bool ok = rep && q_ok && my_local < (uint32_t)n && ((wl & wf) >> (rowc & 31) & 1u);
-            if (RANGE && HALF) {
+            if constexpr (DEBUG) {
+                if (ok) p.out_dists[row] = dist;
+            } else if (RANGE && HALF) {
                 // candidates (NaN included) -> exact distance by the whole warp, the scan's own arithmetic
                 unsigned cm = __ballot_sync(0xffffffffu, ok && !(dist > p.radius + half_margin));
                 while (cm) {
@@ -1065,6 +1076,15 @@ __global__ void __launch_bounds__(scan_max_threads<4>(), 1) scan_kernel_half(con
 template <int METRIC, bool RANGE = false>
 __global__ void __launch_bounds__(256, 1) scan_kernel_half_mma(const ScanParams p) {   // <= 7 consumer warps + 1 producer
     scan_body<METRIC, 1, 16, RANGE, false, 2>(p, nullptr);
+}
+// tests only (mlv_index_debug_half_scan): the approximate distance of every live row, from the consumers above
+template <int METRIC, int R>
+__global__ void __launch_bounds__(scan_max_threads<4>(), 1) scan_kernel_half_debug(const ScanParams p) {
+    scan_body<METRIC, 1, R, true, false, 1, true>(p, nullptr);
+}
+template <int METRIC>
+__global__ void __launch_bounds__(256, 1) scan_kernel_half_mma_debug(const ScanParams p) {
+    scan_body<METRIC, 1, 16, true, false, 2, true>(p, nullptr);
 }
 // one query whose raw values travel in the launch parameters (batch-1 latency path)
 template <int METRIC, int R, bool RANGE>
