@@ -874,13 +874,8 @@ static int search_host_common(mlv_index_t h, const float* queries, uint32_t nq, 
     int64_t* d_rows_out = (int64_t*)h->d_outr.p;
     float* d_dists_out = (float*)((char*)h->d_outr.p + nk * 8);
     int32_t* d_counts_out = (int32_t*)((char*)h->d_outr.p + nk * 12);
-    const uint32_t* filter_dev = nullptr;
-    if (filter_bitmap && h->rows) {
-        const size_t fb = ((h->rows + 31) / 32) * 4;
-        if ((rc = ensure_dev(h, h->d_filter, fb)) != MLV_OK) return rc;
-        CK(h, cudaMemcpyAsync(h->d_filter.p, filter_bitmap, fb, cudaMemcpyHostToDevice, h->stream));
-        filter_dev = (const uint32_t*)h->d_filter.p;
-    }
+    const uint32_t* filter_dev;
+    if ((rc = upload_filter_bitmap(h, filter_bitmap, &filter_dev)) != MLV_OK) return rc;
     memcpy(h->h_stage.p, queries, qbytes);
     CK(h, cudaMemcpyAsync(h->d_qraw.p, h->h_stage.p, qbytes, cudaMemcpyHostToDevice, h->stream));
     if (exchange)
@@ -989,43 +984,15 @@ int mlv_index_range_search_device(mlv_index_t h, const float* queries_dev, uint3
         CK(h, cudaMemsetAsync(out_counts_dev, 0, (size_t)nq * 8, st));
         return MLV_OK;
     }
-    const uint64_t slots = std::max<uint64_t>(max_hits, 1);
+    RangeScan r;
     int rc;
-    // the hit keys of one call: handle-level scratch (one range search at a time per handle)
-    if ((rc = ensure_dev(h, h->d_range, (size_t)nq * slots * 8 + (size_t)nq * 8)) != MLV_OK) return rc;
-    unsigned long long* d_counts = (unsigned long long*)h->d_range.p;
-    uint64_t* d_keys = (uint64_t*)h->d_range.p + nq;
-    CK(h, cudaMemsetAsync(d_counts, 0, (size_t)nq * 8, st));
-    if ((rc = prep_queries(h, queries_dev, nq, st)) != MLV_OK) return rc;
-    Lane* ln = lane_for(h, st);
-    FilterPlan fp;
-    if ((rc = plan_filter(h, ln, filter_bitmap_dev, st, &fp)) != MLV_OK) return rc;
-    ScanCfg c;
-    if ((rc = choose_cfg(h, 1, 1, true, &c, fp.gather != nullptr)) != MLV_OK) return rc;
-    if ((rc = ensure_sched(h, ln)) != MLV_OK) return rc;
-    ScanParams p = scan_params(h, c, fp, ln, 1);
-    bool half = false;   // shadow range scan: half the bytes, candidates re-scored exactly in the kernel (scan_kernel.cuh)
-    {
-        ScanCfg ch;
-        ScanParams ph;
-        if ((rc = half_range_setup(h, fp, ln, st, &half, &ch, &ph)) != MLV_OK) return rc;
-        if (half) {
-            c = ch;
-            p = ph;
-        }
-    }
-    p.radius = radius;
-    p.max_hits = max_hits;
-    for (uint32_t q = 0; q < nq; q++) {
-        p.queries = reinterpret_cast<const float4*>((const float*)ln->d_q.p + (size_t)q * h->ld);
-        p.nq_valid = 1;
-        p.range_counts = d_counts + q;
-        p.range_keys = d_keys + (size_t)q * slots;
-        CK(h, half ? launch_scan_half_range(h, p, c, st) : launch_scan(h, p, c, true, st));
-    }
+    if ((rc = range_setup(h, queries_dev, nq, filter_bitmap_dev, std::max<uint64_t>(max_hits, 1), st, &r)) != MLV_OK) return rc;
+    r.p.radius = radius;
+    r.p.max_hits = max_hits;
+    for (uint32_t q = 0; q < nq; q++) CK(h, launch_range(h, r, q, st));
     CK(h, cudaFuncSetAttribute(range_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(SELECT_MAX_P * 8)));
-    range_finish_kernel<<<nq, SELECT_THREADS, (size_t)SELECT_MAX_P * 8, st>>>(d_keys, d_counts, slots, max_hits, h->row_base, out_dists_dev,
-                                                                            out_rows_dev, (unsigned long long*)out_counts_dev);
+    range_finish_kernel<<<nq, SELECT_THREADS, (size_t)SELECT_MAX_P * 8, st>>>(r.d_keys, r.d_counts, r.slots, max_hits, h->row_base,
+                                                                            out_dists_dev, out_rows_dev, (unsigned long long*)out_counts_dev);
     h->launches++;
     CK(h, cudaGetLastError());
     return MLV_OK;
@@ -1045,20 +1012,15 @@ int mlv_index_range_search(mlv_index_t h, const float* queries, uint32_t nq, flo
     if ((rc = ensure_dev(h, h->d_outd, std::max<size_t>(nh, 1) * 4)) != MLV_OK) return rc;
     if ((rc = ensure_dev(h, h->d_outr, std::max<size_t>(nh, 1) * 8)) != MLV_OK) return rc;
     if ((rc = ensure_dev(h, h->d_outc, (size_t)nq * 8)) != MLV_OK) return rc;
-    const uint32_t* filter_dev = nullptr;
-    if (filter_bitmap) {
-        const size_t fb = ((h->rows + 31) / 32) * 4;
-        if ((rc = ensure_dev(h, h->d_filter, fb)) != MLV_OK) return rc;
-        CK(h, cudaMemcpyAsync(h->d_filter.p, filter_bitmap, fb, cudaMemcpyHostToDevice, h->stream));
-        filter_dev = (const uint32_t*)h->d_filter.p;
-    }
+    const uint32_t* filter_dev;
+    if ((rc = upload_filter_bitmap(h, filter_bitmap, &filter_dev)) != MLV_OK) return rc;
     CK(h, cudaMemcpyAsync(h->d_qraw.p, queries, qbytes, cudaMemcpyHostToDevice, h->stream));
     rc = mlv_index_range_search_device(h, (const float*)h->d_qraw.p, nq, radius, filter_dev, max_hits, (float*)h->d_outd.p,
                                        (int64_t*)h->d_outr.p, (uint64_t*)h->d_outc.p, h->stream);
     if (rc != MLV_OK) return rc;
     CK(h, cudaMemcpyAsync(out_counts, h->d_outc.p, (size_t)nq * 8, cudaMemcpyDeviceToHost, h->stream));
     CK(h, cudaStreamSynchronize(h->stream));
-    h->range_hits_hint = 0;   // how wide this caller's radii are (half_range_setup: the shadow range scan re-scores every hit)
+    h->range_hits_hint = 0;   // how wide this caller's radii are (range_setup: the shadow range scan re-scores every hit)
     for (uint32_t q = 0; q < nq; q++) h->range_hits_hint = std::max<uint64_t>(h->range_hits_hint, out_counts[q]);
     const uint64_t slots = std::max<uint64_t>(max_hits, 1);
     for (uint32_t q = 0; q < nq; q++) {
@@ -1109,43 +1071,19 @@ int mlv_index_range_search_exchange_device(mlv_index_t h, const float* queries_d
         CK(h, cudaGetLastError());
         return MLV_OK;
     }
-    if ((rc = ensure_dev(h, h->d_range, (size_t)nq * share * 8 + (size_t)nq * 8)) != MLV_OK) return rc;
-    unsigned long long* d_counts = (unsigned long long*)h->d_range.p;
-    uint64_t* d_keys = (uint64_t*)h->d_range.p + nq;
-    CK(h, cudaMemsetAsync(d_counts, 0, (size_t)nq * 8, st));
-    if ((rc = prep_queries(h, queries_dev, nq, st)) != MLV_OK) return rc;
-    Lane* ln = lane_for(h, st);
-    FilterPlan fp;
-    if ((rc = plan_filter(h, ln, filter_bitmap_dev, st, &fp)) != MLV_OK) return rc;
-    ScanCfg c;
-    if ((rc = choose_cfg(h, 1, 1, true, &c, fp.gather != nullptr)) != MLV_OK) return rc;
-    if ((rc = ensure_sched(h, ln)) != MLV_OK) return rc;
-    ScanParams p = scan_params(h, c, fp, ln, 1);
-    bool half = false;   // this rank's own choice: its hit list is exact either way
-    {
-        ScanCfg ch;
-        ScanParams ph;
-        if ((rc = half_range_setup(h, fp, ln, st, &half, &ch, &ph)) != MLV_OK) return rc;
-        if (half) {
-            c = ch;
-            p = ph;
-        }
-    }
-    c.smem = std::max(c.smem, (size_t)XCHG_SLOT_KEYS * 8);   // the last CTA sorts / merges up to a slot's worth of keys
-    p.radius = radius;
-    p.max_hits = share;
-    p.fused = 1;
-    p.xchg = x;
+    RangeScan r;
+    if ((rc = range_setup(h, queries_dev, nq, filter_bitmap_dev, share, st, &r)) != MLV_OK) return rc;
+    r.c.smem = std::max(r.c.smem, (size_t)XCHG_SLOT_KEYS * 8);   // the last CTA sorts / merges up to a slot's worth of keys
+    r.p.radius = radius;
+    r.p.max_hits = share;
+    r.p.fused = 1;
+    r.p.xchg = x;
     for (uint32_t q = 0; q < nq; q++) {
-        p.queries = reinterpret_cast<const float4*>((const float*)ln->d_q.p + (size_t)q * h->ld);
-        p.nq_valid = 1;
-        p.range_counts = d_counts + q;
-        p.range_keys = d_keys + (size_t)q * share;
-        p.out_dists = out_dists_dev + (size_t)q * XCHG_SLOT_KEYS;
-        p.out_rows = out_rows_dev + (size_t)q * XCHG_SLOT_KEYS;
-        p.range_out_count = (unsigned long long*)out_counts_dev + q;
-        p.xchg.seq = ++h->xseq;
-        CK(h, half ? launch_scan_half_range(h, p, c, st) : launch_scan(h, p, c, true, st));
+        r.p.out_dists = out_dists_dev + (size_t)q * XCHG_SLOT_KEYS;
+        r.p.out_rows = out_rows_dev + (size_t)q * XCHG_SLOT_KEYS;
+        r.p.range_out_count = (unsigned long long*)out_counts_dev + q;
+        r.p.xchg.seq = ++h->xseq;
+        CK(h, launch_range(h, r, q, st));
     }
     return MLV_OK;
 }
@@ -1166,13 +1104,8 @@ int mlv_index_range_search_exchange(mlv_index_t h, const float* queries, uint32_
     float* hd = (float*)(hc + nq);
     int64_t* hr = (int64_t*)((char*)hd + (size_t)nq * XCHG_SLOT_KEYS * 4);
     char* hq = (char*)hr + (size_t)nq * XCHG_SLOT_KEYS * 8;
-    const uint32_t* filter_dev = nullptr;
-    if (filter_bitmap && h->rows) {
-        const size_t fb = ((h->rows + 31) / 32) * 4;
-        if ((rc = ensure_dev(h, h->d_filter, fb)) != MLV_OK) return rc;
-        CK(h, cudaMemcpyAsync(h->d_filter.p, filter_bitmap, fb, cudaMemcpyHostToDevice, h->stream));
-        filter_dev = (const uint32_t*)h->d_filter.p;
-    }
+    const uint32_t* filter_dev;
+    if ((rc = upload_filter_bitmap(h, filter_bitmap, &filter_dev)) != MLV_OK) return rc;
     memcpy(hq, queries, qbytes);
     CK(h, cudaMemcpyAsync(h->d_qraw.p, hq, qbytes, cudaMemcpyHostToDevice, h->stream));
     rc = mlv_index_range_search_exchange_device(h, (const float*)h->d_qraw.p, nq, radius, filter_dev, hd, hr, hc, h->stream);
@@ -1412,24 +1345,13 @@ int mlv_index_debug_half_scan(mlv_index_t h, const float* query, float* out_appr
     if ((rc = ensure_dev(h, h->d_qraw, (size_t)h->dim * 4)) != MLV_OK) return rc;
     CK(h, cudaMemcpyAsync(h->d_qraw.p, query, (size_t)h->dim * 4, cudaMemcpyHostToDevice, st));
     if ((rc = prep_queries(h, (const float*)h->d_qraw.p, 1, st)) != MLV_OK) return rc;
-    if (h->metric != MLV_COSINE && (rc = ensure_row_norms(h, st)) != MLV_OK) return rc;
     bool usable = false;
-    if ((rc = ensure_f16_shadow(h, st, &usable)) != MLV_OK) return rc;
+    if ((rc = ensure_shadow(h, st, &usable)) != MLV_OK) return rc;
     if (!usable) return fail(h, MLV_E_NOMEM, "no room for the fp16 shadow");
-    const int half_kind = (f16_ld(h) % 64 == 0 && h->tune_scan_half_mma != 0) ? 2 : 1;   // search_prepared's choice
     ScanCfg c;
-    if ((rc = choose_cfg(h, 1, 1, true, &c, false, half_kind)) != MLV_OK) return rc;
-    ScanParams p = scan_params(h, c, FilterPlan{}, ln, 1);
+    if ((rc = choose_cfg(h, 1, 1, true, &c, false, shadow_consumers(h))) != MLV_OK) return rc;
+    ScanParams p = shadow_params(h, c, FilterPlan{}, ln, 1);
     p.sched = nullptr;
-    p.rows = reinterpret_cast<const float4*>(h->d_rows16.p);
-    p.ld4 = f16_ld(h) / 8;
-    p.rows_exact = reinterpret_cast<const float4*>(h->d_rows);
-    p.ld4_exact = h->ld / 4;
-    p.half_state = (const uint32_t*)h->d_f16st.p;
-    p.row_norms = h->metric == MLV_L2 ? (const float*)h->d_norms.p : nullptr;
-    p.max_norm2_bits = h->metric == MLV_COSINE ? nullptr : (const uint32_t*)h->d_maxn2.p;
-    p.delta_rel = gemm_delta_rel_f16_host(h->metric == MLV_L2, h->ld);
-    p.cosine = h->metric == MLV_COSINE;
     p.queries = reinterpret_cast<const float4*>(ln->d_q.p);
     p.nq_valid = 1;
     // [rows] approximate distances (+inf where the kernel stores nothing) | |q|^2, 2^-s 2^-t, scale

@@ -237,3 +237,32 @@ def test_shadow_range_scan_returns_the_fp32_hit_lists(space, dim):
         both(float(d10[2, 15]))
         both(float(d10[2, 15]))                            # ... and the shadow has been rebuilt
     s.close()
+
+
+def test_timing_records_one_event_pair_per_search_and_per_range_query():
+    """scan_time_ms averages searches, not launches: a shadow-pair search (the shadow scan and the conditional fp32 launch
+    behind it) records one event pair, as does an fp32 single query; a range search records one per query, over the
+    shadow or over the fp32 rows."""
+    n, dim, k = 40_000, 128, 10
+    X = synthetic.rows(97, 0, n, dim, scaled=True)
+    Q = synthetic.queries(98, 3, dim)
+    s = _shard(dim, "l2")
+    s.add(X)
+    s.set_tuning("scan_half", 0)
+    radius = float(s.search(Q, 5)[0][:, 4].min())      # at most ~5 hits per query
+    s.set_timing(True)
+    s.scan_time_ms()
+    for half in (1, 0):
+        s.set_tuning("scan_half", half)
+        before = s.gemm_stats()["half_scan_queries"]
+        s.search(Q[:1], k)
+        assert s.gemm_stats()["half_scan_queries"] - before == half
+        ms, pairs = s.scan_time_ms()
+        assert pairs == 1 and ms > 0, (half, pairs, ms)
+    for half in (1, 0):
+        s.set_tuning("scan_half", half)
+        s.range_search(Q, radius)
+        ms, pairs = s.scan_time_ms()
+        assert pairs == 3 and ms > 0, (half, pairs, ms)
+    s.set_timing(False)
+    s.close()
