@@ -422,6 +422,30 @@ int mlv_index_gemm_stats(mlv_index_t h, mlv_gemm_stats_t *out);
  */
 int mlv_index_debug_gemm(mlv_index_t h, const float *queries, uint32_t nq, float *out_approx);
 /*
+ * Debug / selection tests: GEMM rounds over every stored row as a batch search runs them -- the production kernels
+ * (gemm_topk_kernel or the CTA-pair kernel, each round optionally followed by refine_kernel) -- with the tier, kernel,
+ * grid, initial thresholds, candidate capacity and round schedule chosen by the caller.  Returns the raw buffers:
+ * out_keys[nq, cap] (slot j of query i is meaningful for j < min(out_counts[i], cap); keys are (distance, row) packed
+ * as in gemm_kernel.cuh: f32_orderable(distance) << 32 | row), out_counts[nq] (uncapped: hits beyond `cap` are
+ * counted, not stored), out_thr[nq] and out_flags[nq] (refine_kernel: bit 0 overflow, bit 2 starved / failed
+ * prediction), and *out_pad_count, what the padding queries of the last query tile appended (0 when correct).
+ * thresholds[nq] = the initial per-query thresholds (NULL = +inf; padding queries keep -inf); filter_bitmap =
+ * ceil(rows / 32) words or NULL.  Any output pointer may be NULL.  rows >= 1, dim >= 32.
+ */
+typedef struct mlv_gemm_rounds_cfg {
+    uint32_t passes;                /* 1 = one-pass TF32, 2 = fp16 shadow, 3 = 3xTF32 */
+    uint32_t bn;                    /* single-tile kernel with 64 / 128 / 256 queries per tile; 0 = CTA-pair kernel (passes 1, 2) */
+    uint32_t max_ctas;              /* grid limit, 0 = the grid a search launches (pairs: rounded down to an even count, >= 2) */
+    uint32_t cap;                   /* candidate slots per query (>= 1; a power of two <= 8192 when kprime > 0) */
+    uint32_t kprime;                /* refine_kernel keeps this many after every round; 0 = no refine (raw emission) */
+    uint32_t n_rounds;              /* >= 1 */
+    const uint32_t *round_end;      /* [n_rounds] row tile (128 rows) each round ends before, ascending, the last <= ceil(rows / 128) */
+    const uint32_t *round_jrank;    /* [n_rounds] rank refine_kernel sets the threshold from, 1..kprime (unused when kprime is 0) */
+} mlv_gemm_rounds_cfg_t;
+int mlv_index_debug_gemm_rounds(mlv_index_t h, const float *queries, uint32_t nq, const float *thresholds,
+                                const uint32_t *filter_bitmap, const mlv_gemm_rounds_cfg_t *cfg, uint64_t *out_keys,
+                                uint32_t *out_counts, float *out_thr, uint32_t *out_flags, uint64_t *out_pad_count);
+/*
  * Debug / bound tests: the APPROXIMATE distances the shadow scan's consumers compute for ONE host query against every
  * stored row (the same consumer code: FMA or tensor-core consumers, whichever "scan_half_mma" and the row length select
  * for a search), before any re-scoring: out_approx[rows], +inf for tombstoned rows.  *out_info receives what the

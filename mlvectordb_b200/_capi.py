@@ -65,6 +65,20 @@ class HalfScanDebug(C.Structure):
     ]
 
 
+class GemmRoundsCfg(C.Structure):
+    """``mlv_gemm_rounds_cfg_t``"""
+    _fields_ = [
+        ("passes", C.c_uint32),
+        ("bn", C.c_uint32),
+        ("max_ctas", C.c_uint32),
+        ("cap", C.c_uint32),
+        ("kprime", C.c_uint32),
+        ("n_rounds", C.c_uint32),
+        ("round_end", C.POINTER(C.c_uint32)),
+        ("round_jrank", C.POINTER(C.c_uint32)),
+    ]
+
+
 class Predicate(C.Structure):
     """``mlv_predicate_t``"""
     _fields_ = [("column", C.c_uint32), ("op", C.c_int32), ("a", C.c_int32), ("b", C.c_int32)]
@@ -146,6 +160,8 @@ SIGNATURES = {
     "mlv_index_gemm_stats": (C.c_int, [_h, C.POINTER(GemmStats)]),
     "mlv_index_debug_gemm": (C.c_int, [_h, C.c_void_p, C.c_uint32, C.c_void_p]),
     "mlv_index_debug_half_scan": (C.c_int, [_h, C.c_void_p, C.c_void_p, C.POINTER(HalfScanDebug)]),
+    "mlv_index_debug_gemm_rounds": (C.c_int, [_h, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.POINTER(GemmRoundsCfg),
+                                              C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, _u64p]),
 }
 
 _lib = None

@@ -1262,76 +1262,34 @@ int mlv_index_debug_gemm(mlv_index_t h, const float* queries, uint32_t nq, float
     if (!h || !queries || !out_approx || nq == 0) return fail(h, MLV_E_INVALID, "bad argument");
     if (h->rows == 0 || h->rows > SELECT_MAX_P || h->ld < (uint32_t)GEMM_BK) return fail(h, MLV_E_UNSUPPORTED, "debug_gemm needs 1..8192 rows and dim >= 32");
     DeviceGuard g(h->device);
-    cudaStream_t st = h->stream;
-    int rc;
-    const uint32_t ld = h->ld;
-    const size_t qbytes = (size_t)nq * h->dim * 4;
-    if ((rc = ensure_dev(h, h->d_qraw, qbytes)) != MLV_OK) return rc;
-    CK(h, cudaMemcpyAsync(h->d_qraw.p, queries, qbytes, cudaMemcpyHostToDevice, st));
-    if ((rc = prep_queries(h, (const float*)h->d_qraw.p, nq, st)) != MLV_OK) return rc;
-    if (h->metric != MLV_COSINE && (rc = ensure_row_norms(h, st)) != MLV_OK) return rc;
-    const uint32_t GEMM_BN = gemm_tile_width(h, nq);
-    const uint32_t nq_pad = (nq + GEMM_BN - 1) / GEMM_BN * GEMM_BN;
-    const uint32_t cap = pow2_ceil((uint32_t)h->rows);
-    const size_t qmat = (size_t)nq_pad * ld * 4;
-    if ((rc = ensure_dev(h, h->d_gq, 2 * qmat + (size_t)nq_pad * 20)) != MLV_OK) return rc;
-    if ((rc = ensure_dev(h, h->d_cand, (size_t)nq_pad * cap * 8)) != MLV_OK) return rc;
-    float* qhi = (float*)h->d_gq.p;
-    float* qlo = qhi + (size_t)nq_pad * ld;
-    float* qn = qlo + (size_t)nq_pad * ld;
-    float* thr = qn + nq_pad;
-    uint32_t* cnt = (uint32_t*)(thr + nq_pad);
-    uint32_t* flags = cnt + nq_pad;
-    uint32_t* sorted_n = flags + nq_pad;
-    const int passes = h->tune_gemm_passes == 1 ? 1 : (h->tune_gemm_passes == GEMM_TIER_F16 ? GEMM_TIER_F16 : 3);   // which tier's distances
-    const bool half = passes == GEMM_TIER_F16;
-    const uint32_t ld16 = f16_ld(h);
-    if (half) {
-        bool usable = false;
-        if ((rc = ensure_f16_shadow(h, st, &usable)) != MLV_OK) return rc;
-        if (!usable) return fail(h, MLV_E_NOMEM, "no room for the fp16 shadow");
-        split_queries_f16_kernel<<<(nq_pad + 7) / 8, 256, 0, st>>>((const float*)lane_for(h, st)->d_q.p, (__half*)qhi, qlo, qn, thr, cnt, flags,
-                                                                  sorted_n, nq, nq_pad, ld, ld16);
-    } else {
-        split_queries_kernel<<<(nq_pad + 7) / 8, 256, 0, st>>>((const float*)lane_for(h, st)->d_q.p, qhi, qlo, qn, thr, cnt, flags, sorted_n, nq, nq_pad, ld);
-    }
-    CK(h, cudaGetLastError());
-    CUtensorMap mx, mqh, mql;
-    if ((rc = make_tile_map(h, &mx, half ? h->d_rows16.p : (const void*)h->d_rows, h->rows, GEMM_BM, half)) != MLV_OK) return rc;
-    if ((rc = make_tile_map(h, &mqh, qhi, nq_pad, GEMM_BN, half)) != MLV_OK) return rc;
-    if ((rc = make_tile_map(h, &mql, half ? qhi : qlo, nq_pad, GEMM_BN, half)) != MLV_OK) return rc;
-    GemmParams gp{};
-    gp.n_rows = (uint32_t)h->rows;
-    gp.nq = nq;
-    gp.n_qtiles = nq_pad / GEMM_BN;
-    gp.n_kchunks = half ? (ld16 + 2 * GEMM_BK - 1) / (2 * GEMM_BK) : (ld + GEMM_BK - 1) / GEMM_BK;
-    gp.x_unscale = (const float*)h->d_f16st.p;
-    gp.q_unscale = qlo;
-    gp.row_norms = h->metric == MLV_L2 ? (const float*)h->d_norms.p : nullptr;
-    gp.q_norms = qn;
-    gp.thr = thr;
-    gp.live = h->n_deleted ? h->d_live : nullptr;
-    gp.cand = (uint64_t*)h->d_cand.p;
-    gp.cand_cnt = cnt;
-    gp.cap = cap;
-    gp.row_tile0 = 0;
-    gp.row_tile1 = (uint32_t)((h->rows + GEMM_BM - 1) / GEMM_BM);
-    const int grid = (int)std::min<uint64_t>((uint64_t)gp.row_tile1 * gp.n_qtiles, (uint64_t)h->sm_count);
-    CK(h, h->metric == MLV_L2 ? launch_gemm_t<METRIC_L2>(mx, mqh, mql, gp, grid, st, (int)GEMM_BN, passes)
-                              : launch_gemm_t<METRIC_IP>(mx, mqh, mql, gp, grid, st, (int)GEMM_BN, passes));
-    h->launches += 3;
-    std::vector<uint64_t> keys((size_t)nq * cap);
+    // one round over every row tile at threshold +inf: each live row is a candidate of every query
+    const uint32_t tiles = (uint32_t)((h->rows + GEMM_BM - 1) / GEMM_BM);
+    mlv_gemm_rounds_cfg_t c{};
+    c.passes = h->tune_gemm_passes == 1 ? 1u : (h->tune_gemm_passes == GEMM_TIER_F16 ? (uint32_t)GEMM_TIER_F16 : 3u);   // which tier's distances
+    c.bn = gemm_tile_width(h, nq);
+    c.cap = pow2_ceil((uint32_t)h->rows);
+    c.n_rounds = 1;
+    c.round_end = &tiles;
+    std::vector<uint64_t> keys((size_t)nq * c.cap);
     std::vector<uint32_t> counts(nq);
-    CK(h, cudaMemcpyAsync(keys.data(), h->d_cand.p, keys.size() * 8, cudaMemcpyDeviceToHost, st));
-    CK(h, cudaMemcpyAsync(counts.data(), cnt, (size_t)nq * 4, cudaMemcpyDeviceToHost, st));
-    CK(h, cudaStreamSynchronize(st));
+    int rc;
+    if ((rc = gemm_rounds_debug(h, queries, nq, nullptr, nullptr, c, keys.data(), counts.data(), nullptr, nullptr, nullptr)) != MLV_OK) return rc;
     for (size_t i = 0; i < (size_t)nq * h->rows; i++) out_approx[i] = std::numeric_limits<float>::quiet_NaN();
     for (uint32_t q = 0; q < nq; q++)
-        for (uint32_t i = 0; i < std::min(counts[q], cap); i++) {
-            const uint64_t key = keys[(size_t)q * cap + i];
+        for (uint32_t i = 0; i < std::min(counts[q], c.cap); i++) {
+            const uint64_t key = keys[(size_t)q * c.cap + i];
             if (key_row(key) < h->rows) out_approx[(size_t)q * h->rows + key_row(key)] = key_dist(key);
         }
     return MLV_OK;
+}
+
+int mlv_index_debug_gemm_rounds(mlv_index_t h, const float* queries, uint32_t nq, const float* thresholds, const uint32_t* filter_bitmap,
+                                const mlv_gemm_rounds_cfg_t* cfg, uint64_t* out_keys, uint32_t* out_counts, float* out_thr,
+                                uint32_t* out_flags, uint64_t* out_pad_count) {
+    if (!h) return MLV_E_INVALID;
+    if (!cfg) return fail(h, MLV_E_INVALID, "bad argument");
+    DeviceGuard g(h->device);
+    return gemm_rounds_debug(h, queries, nq, thresholds, filter_bitmap, *cfg, out_keys, out_counts, out_thr, out_flags, out_pad_count);
 }
 
 int mlv_index_debug_half_scan(mlv_index_t h, const float* query, float* out_approx, mlv_half_scan_debug_t* out_info) {

@@ -39,6 +39,21 @@ def pack_bitmap(mask: np.ndarray) -> np.ndarray:
     return np.packbits(mask, bitorder="little").view(np.uint32)
 
 
+def key_parts(keys: np.ndarray) -> Tuple[np.ndarray, np.ndarray]:
+    """Candidate keys (uint64: f32_orderable(distance) << 32 | row, csrc/common.cuh) -> (distance float32, row uint32)."""
+    k = np.asarray(keys, dtype=np.uint64)
+    o = (k >> np.uint64(32)).astype(np.uint32)
+    bits = np.where(o & np.uint32(0x80000000), o & np.uint32(0x7FFFFFFF), ~o).astype(np.uint32)
+    return bits.view(np.float32), (k & np.uint64(0xFFFFFFFF)).astype(np.uint32)
+
+
+def make_keys(dist: np.ndarray, rows: np.ndarray) -> np.ndarray:
+    """(distance float32, row) -> the kernels' uint64 keys, whose unsigned order is (distance, row) ascending."""
+    b = np.ascontiguousarray(dist, dtype=np.float32).view(np.uint32)
+    o = np.where(b & np.uint32(0x80000000), ~b, b | np.uint32(0x80000000)).astype(np.uint64)
+    return (o << np.uint64(32)) | np.asarray(rows, dtype=np.uint64)
+
+
 class DeviceShard:
     def __init__(self, dim: int, space: str = "l2", capacity: int = 0, device: int = 0, row_base: int = 0):
         self.space = canonical_space(space)
@@ -353,6 +368,33 @@ class DeviceShard:
         out = np.empty((q.shape[0], self.rows), dtype=np.float32)
         self._ck(self._lib.mlv_index_debug_gemm(self._h, q.ctypes.data_as(C.c_void_p), q.shape[0],
                                                 out.ctypes.data_as(C.c_void_p)))
+        return out
+
+    def debug_gemm_rounds(self, queries: np.ndarray, passes: int, bn: int, cap: int, rounds=None, kprime: int = 0,
+                          thresholds: Optional[np.ndarray] = None, mask: Optional[np.ndarray] = None, max_ctas: int = 0) -> dict:
+        """GEMM rounds as a batch search runs them (``mlv_index_debug_gemm_rounds``; tests only).  bn 64 / 128 / 256 =
+        single-tile kernel, 0 = CTA pair; rounds = [(end_tile, jrank), ...] (default: one round over every tile);
+        thresholds[nq] initial (None = +inf); mask = bool[rows] filter.  -> dict of keys [nq, cap] uint64, counts
+        (uncapped), thr, flags, pad_count."""
+        q = np.ascontiguousarray(queries, dtype=np.float32).reshape(-1, self.dim)
+        nq = q.shape[0]
+        if rounds is None:
+            rounds = [(-(-self.rows // 128), kprime)]
+        ends = np.ascontiguousarray([r[0] for r in rounds], dtype=np.uint32)
+        jr = np.ascontiguousarray([r[1] for r in rounds], dtype=np.uint32)
+        cfg = _capi.GemmRoundsCfg(int(passes), int(bn), int(max_ctas), int(cap), int(kprime), len(rounds),
+                                  ends.ctypes.data_as(C.POINTER(C.c_uint32)), jr.ctypes.data_as(C.POINTER(C.c_uint32)))
+        thr = None if thresholds is None else np.ascontiguousarray(thresholds, dtype=np.float32).reshape(nq)
+        bm = None if mask is None else pack_bitmap(mask)
+        out = {"keys": np.empty((nq, int(cap)), np.uint64), "counts": np.empty(nq, np.uint32),
+               "thr": np.empty(nq, np.float32), "flags": np.empty(nq, np.uint32)}
+        pad = C.c_uint64()
+        self._ck(self._lib.mlv_index_debug_gemm_rounds(
+            self._h, q.ctypes.data_as(C.c_void_p), nq, None if thr is None else thr.ctypes.data_as(C.c_void_p),
+            None if bm is None else bm.ctypes.data_as(C.c_void_p), C.byref(cfg), out["keys"].ctypes.data_as(C.c_void_p),
+            out["counts"].ctypes.data_as(C.c_void_p), out["thr"].ctypes.data_as(C.c_void_p),
+            out["flags"].ctypes.data_as(C.c_void_p), C.byref(pad)))
+        out["pad_count"] = int(pad.value)
         return out
 
     def debug_half_scan(self, query: np.ndarray) -> Tuple[np.ndarray, dict]:

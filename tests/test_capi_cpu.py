@@ -116,3 +116,28 @@ def test_every_tuning_key_is_documented_in_the_header():
     keys = sorted(set(re.findall(r'k == "([a-z0-9_]+)"', src)))
     assert len(keys) >= 20
     assert [k for k in keys if f'"{k}"' not in hdr] == []
+
+
+def test_candidate_key_decoder_inverts_the_kernels_encoding():
+    """key_parts is the inverse of f32_orderable (csrc/common.cuh): keys order as (distance, row) and decode bit-exactly,
+    including +-0, +-inf, NaN, subnormals and negative values."""
+    from mlvectordb_b200.shard import key_parts, make_keys
+    tiny = np.float32(1.4e-45)
+    vals = np.array([-np.inf, -3.4e38, -1.5, -tiny, -0.0, 0.0, tiny, 1e-40, 1.0, 3.4e38, np.inf, np.nan], np.float32)
+    rows = np.arange(len(vals), dtype=np.uint32) * np.uint32(977)
+    keys = make_keys(vals, rows)
+    # f32_orderable: sign set -> all bits flipped, else the sign bit set
+    hi = (keys >> np.uint64(32)).astype(np.uint32)
+    assert hi[4] == 0x7FFFFFFF and hi[5] == 0x80000000 and hi[0] == 0x007FFFFF and hi[10] == 0xFF800000
+    d, r = key_parts(keys)
+    assert np.array_equal(d.view(np.uint32), vals.view(np.uint32)) and np.array_equal(r, rows)
+    assert (np.diff(keys.astype(np.uint64)) > 0).all(), "key order is not the distance order"   # vals ascend, NaN last
+    rng = np.random.default_rng(0)
+    bits = rng.integers(0, 2 ** 32, 10_000, dtype=np.uint64).astype(np.uint32)
+    rr = rng.integers(0, 2 ** 32, 10_000, dtype=np.uint64).astype(np.uint32)
+    d, r = key_parts(make_keys(bits.view(np.float32), rr))
+    assert np.array_equal(d.view(np.uint32), bits) and np.array_equal(r, rr)
+    fin = ~np.isnan(bits.view(np.float32))
+    k = make_keys(bits.view(np.float32)[fin], np.zeros(fin.sum(), np.uint32))
+    o = np.argsort(k, kind="stable")
+    assert (np.diff(bits.view(np.float32)[fin][o].astype(np.float64)) >= 0).all()
