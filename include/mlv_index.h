@@ -29,7 +29,7 @@
 extern "C" {
 #endif
 
-#define MLV_ABI_VERSION 5
+#define MLV_ABI_VERSION 6
 
 typedef struct mlv_index *mlv_index_t;
 
@@ -354,7 +354,7 @@ int mlv_index_scan_time_ms(mlv_index_t h, double *total_ms, uint64_t *launches);
  * final select, 0 = separate select kernel), "gather" (-1 auto, 0 = filters stream every row and mask,
  * 1 = filters always gather; the tensor-core path compacts the passing rows accordingly), "staged_upload"
  * (1 = bulk mlv_index_add through two pinned chunks filled by worker threads, 0 = plain copy), "fast_host" (1 = single-query
- * mlv_index_search takes the one-launch latency path, 0 = always staged), "scan_half" / "scan_half_mma" (below), and the
+ * mlv_index_search takes the one-launch latency path, 0 = always staged), "scan_half" / "scan_half_mma" / "scan_q8" (below), and the
  * tensor-core keys listed at mlv_index_gemm_stats}.  Results never depend on these.
  *
  * Shadow scan ("scan_half": -1 auto = matrices of 256 MB and more, 0 never, 1 whenever the shape allows).  A SINGLE
@@ -370,7 +370,15 @@ int mlv_index_scan_time_ms(mlv_index_t h, double *total_ms, uint64_t *launches);
  * when they are at least 256 bytes and the row list is worth 1 GB of fp32 rows; 0 = gathered scans read the fp32 rows.  A shadow that certifies less than half of its searches sits out 64, 128, ... searches.  In an exchange
  * search every rank issues the same two launches whether or not it has a shadow to read (the ranks agree on the
  * certificate through the exchange itself), so "scan_half" must be 0 on all ranks or on none.
- * mlv_index_gemm_stats reports half_scan_queries / half_scan_uncertified.
+ * Int8 shadow ("scan_q8": -1 auto, 0 never, 1 whatever the matrix size).  With "scan_half" auto (-1), a shadow scan of a
+ * full (not gathered) matrix of 256 MB and more reads an int8 shadow instead: one int8 digit per element and one scale per
+ * row (+ 25 % device memory, built and kept up to date like the fp16 one), a quarter of the fp32 bytes.  It keeps 64
+ * candidates and certifies them against its own error bound (q8_delta in scan_kernel.cuh); the fp32 launch behind it
+ * works as above, so the results are again the fp32 scan's bit for bit.  An int8 shadow that certifies less than half of
+ * its searches sits out 64, 128, ... searches while the fp16 shadow answers.  "scan_half" = 1 always reads the fp16 shadow.
+ * Each rank of an exchange search picks its own shadow.
+ * mlv_index_gemm_stats reports half_scan_queries / half_scan_uncertified (both shadows) and q8_scan_queries /
+ * q8_scan_uncertified (the int8 one alone).
  */
 int mlv_index_set_tuning(mlv_index_t h, const char *key, int value);
 /*
@@ -413,6 +421,8 @@ typedef struct mlv_gemm_stats {
     uint64_t mispredicted_queries; /* queries whose predicted thresholds failed the final check ("gemm_predict"); answered by the next tier */
     uint64_t half_scan_queries;    /* single queries answered through the shadow scan ("scan_half"; not a tensor-core path, counted here for one stats call) */
     uint64_t half_scan_uncertified; /* of those, re-run by the fp32 scan launch queued behind (certificate failed / shadow overflowed) */
+    uint64_t q8_scan_queries;      /* of half_scan_queries, those whose shadow scan read the int8 shadow ("scan_q8") */
+    uint64_t q8_scan_uncertified;  /* of those, re-run by the fp32 scan launch queued behind */
 } mlv_gemm_stats_t;
 int mlv_index_gemm_stats(mlv_index_t h, mlv_gemm_stats_t *out);
 /*
@@ -462,6 +472,19 @@ typedef struct mlv_half_scan_debug {
     uint32_t consumers; /* 1 = FMA consumers, 2 = tensor-core consumers (mma.sync) */
 } mlv_half_scan_debug_t;
 int mlv_index_debug_half_scan(mlv_index_t h, const float *query, float *out_approx, mlv_half_scan_debug_t *out_info);
+/*
+ * Debug / bound tests: the same for the int8 shadow's consumers (scan_kernel_q8): out_approx[rows] (+inf for tombstoned
+ * rows) and what its certificate uses.  1 <= rows <= 8192.
+ */
+typedef struct mlv_q8_scan_debug {
+    float delta;        /* bound on |approx - exact| for every row (scan_kernel.cuh, q8_delta), as the kernel computed it */
+    float q_norm2;      /* |q|^2 of the prepared query, as the kernel computed it */
+    float q_scale;      /* t: the query is t (h + l / 254) + r with int8 digits h, l */
+    float max_norm2;    /* largest |x|^2 of the rows (0 for cosine: unit rows) */
+    float e_max;        /* E: largest bound on |x - s_x x^| over the rows */
+    uint32_t ld8;       /* bytes per row of the int8 shadow */
+} mlv_q8_scan_debug_t;
+int mlv_index_debug_q8_scan(mlv_index_t h, const float *query, float *out_approx, mlv_q8_scan_debug_t *out_info);
 /* Kernels launched by this handle since creation (scan + select + maintenance). */
 int mlv_index_kernel_launches(mlv_index_t h, uint64_t *launches);
 

@@ -17,7 +17,7 @@ MLV_OK = 0
 MLV_E_INVALID, MLV_E_CUDA, MLV_E_NOMEM, MLV_E_UNSUPPORTED, MLV_E_NO_DEVICE = 1, 2, 3, 4, 5
 MLV_MAX_K = 1024
 METRIC_CODE = {"l2": 0, "ip": 1, "cosine": 2}
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 
 class IndexInfo(C.Structure):
@@ -48,6 +48,8 @@ class GemmStats(C.Structure):
         ("mispredicted_queries", C.c_uint64),
         ("half_scan_queries", C.c_uint64),
         ("half_scan_uncertified", C.c_uint64),
+        ("q8_scan_queries", C.c_uint64),
+        ("q8_scan_uncertified", C.c_uint64),
     ]
 
 
@@ -62,6 +64,18 @@ class HalfScanDebug(C.Structure):
         ("q_unscale", C.c_float),
         ("overflow", C.c_uint32),
         ("consumers", C.c_uint32),
+    ]
+
+
+class Q8ScanDebug(C.Structure):
+    """``mlv_q8_scan_debug_t``"""
+    _fields_ = [
+        ("delta", C.c_float),
+        ("q_norm2", C.c_float),
+        ("q_scale", C.c_float),
+        ("max_norm2", C.c_float),
+        ("e_max", C.c_float),
+        ("ld8", C.c_uint32),
     ]
 
 
@@ -160,6 +174,7 @@ SIGNATURES = {
     "mlv_index_gemm_stats": (C.c_int, [_h, C.POINTER(GemmStats)]),
     "mlv_index_debug_gemm": (C.c_int, [_h, C.c_void_p, C.c_uint32, C.c_void_p]),
     "mlv_index_debug_half_scan": (C.c_int, [_h, C.c_void_p, C.c_void_p, C.POINTER(HalfScanDebug)]),
+    "mlv_index_debug_q8_scan": (C.c_int, [_h, C.c_void_p, C.c_void_p, C.POINTER(Q8ScanDebug)]),
     "mlv_index_debug_gemm_rounds": (C.c_int, [_h, C.c_void_p, C.c_uint32, C.c_void_p, C.c_void_p, C.POINTER(GemmRoundsCfg),
                                               C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, _u64p]),
 }

@@ -97,6 +97,7 @@ __host__ __device__ inline float gemm_delta_rel_f16(bool l2, uint32_t d) {
     const float e = 9.765625e-4f * (1.0f + 2.44140625e-4f) + (float)d * 2.384185791015625e-7f + 9.5367431640625e-7f;
     return l2 ? 0.5f * e : e;
 }
+// The int8 shadow's bound (q8_delta) is in scan_kernel.cuh, next to the kernel that uses it.
 
 struct GemmParams {
     uint32_t n_rows;
@@ -835,6 +836,51 @@ __global__ void convert_rows_f16_kernel(const float* __restrict__ rows, uint64_t
         reinterpret_cast<__half2*>(out + (first + r) * ld16)[c >> 1] = __floats2half2_rn(a, b);
     }
     if (over) st[2] = 1;
+}
+// ---- int8 shadow of the rows (scan_kernel_q8, see q8_delta in scan_kernel.cuh) ------------------------------------
+// rows [first, first + n) -> int8 digits x^ = rint(x / s_x) with s_x = max |x| / 127 (one scale per row, so appended rows
+// cannot overflow), ld8 bytes per row (zero padded).  sx[row] = s_x; *e_bits = max over the rows of e_x >= |x - s_x x^|_2
+// (float bits: non-negative floats order as uints, a NaN row wins and leaves every query uncertified).  One warp per row.
+__global__ void convert_rows_q8_kernel(const float* __restrict__ rows, uint64_t first, uint64_t n, uint32_t ld, uint32_t ld8,
+                                       int8_t* __restrict__ out, float* __restrict__ sx, uint32_t* e_bits) {
+    const uint64_t w = (uint64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+    const int lane = threadIdx.x & 31;
+    if (w >= n) return;
+    const float4* src = reinterpret_cast<const float4*>(rows + (first + w) * ld);
+    const uint32_t ld4 = ld >> 2;
+    float m = 0.f;
+    for (uint32_t j = lane; j < ld4; j += 32) {
+        const float4 x = src[j];
+        m = fmaxf(m, fmaxf(fmaxf(fabsf(x.x), fabsf(x.y)), fmaxf(fabsf(x.z), fabsf(x.w))));
+    }
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, off));
+    const float s = m / 127.0f;
+    const float inv = m > 0.f ? 127.0f / m : 0.f;
+    uint32_t* dst = reinterpret_cast<uint32_t*>(out + (first + w) * ld8);
+    float ss = 0.f;
+    for (uint32_t j = lane; j < ld8 / 4; j += 32) {
+        const float4 x = j < ld4 ? src[j] : make_float4(0.f, 0.f, 0.f, 0.f);
+        const float v[4] = {x.x, x.y, x.z, x.w};
+        uint32_t packed = 0;
+#pragma unroll
+        for (int i = 0; i < 4; i++) {
+            const float dq = fminf(fmaxf(rintf(v[i] * inv), -127.f), 127.f);
+            const float r = fmaf(-s, dq, v[i]);
+            ss = fmaf(r, r, ss);
+            packed |= ((uint32_t)(int32_t)dq & 0xffu) << (8 * i);
+        }
+        dst[j] = packed;
+    }
+#pragma unroll
+    for (int off = 16; off >= 1; off >>= 1) ss += __shfl_xor_sync(0xffffffffu, ss, off);
+    if (lane == 0) {
+        // rounded up: each residual is one fma (relative 2^-24), the fp32 sum of ld squares is off by <= ld 2^-23 of itself,
+        // squares below the normal range add < 2^-60 in total
+        const float e = sqrtf(ss) * (1.0f + (float)(ld + 4) * 2.384185791015625e-7f) + 8.673617379884035e-19f;
+        sx[first + w] = s;
+        atomicMax(e_bits, __float_as_uint(e));
+    }
 }
 // Prepared queries [nq, ld] -> halves of q * 2^sq [nq_pad, ld16] (pad rows / columns zero), 2^-sq, |q|^2, initial thresholds,
 // cleared counters and flags.  One warp per (padded) query.

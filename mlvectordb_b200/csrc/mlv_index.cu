@@ -117,6 +117,7 @@ int mlv_index_create(uint32_t dim, int metric, uint64_t capacity_hint, int devic
     h->tune_scan_half = env_int("MLV_SCAN_HALF", h->tune_scan_half);
     h->tune_scan_half_mma = env_int("MLV_SCAN_HALF_MMA", h->tune_scan_half_mma);
     h->tune_scan_half_gather = env_int("MLV_SCAN_HALF_GATHER", h->tune_scan_half_gather);
+    h->tune_scan_q8 = env_int("MLV_SCAN_Q8", h->tune_scan_q8);
     DeviceGuard g(device);
     cudaDeviceProp prop;
     cudaError_t e = g.ok ? cudaGetDeviceProperties(&prop, device) : cudaErrorInvalidDevice;
@@ -153,7 +154,8 @@ int mlv_index_destroy(mlv_index_t h) {
     if (h->d_rows) cudaFree(h->d_rows);
     if (h->d_live) cudaFree(h->d_live);
     for (DevBuf* b : {&h->d_qraw, &h->d_filter, &h->d_outd, &h->d_outr, &h->d_outc, &h->d_misc, &h->d_range, &h->d_timeline,
-                      &h->d_norms, &h->d_gq, &h->d_cand, &h->d_maxn2, &h->d_sub, &h->d_gx, &h->d_rows16, &h->d_f16st, &h->d_gx16, &h->d_half_stats})
+                      &h->d_norms, &h->d_gq, &h->d_cand, &h->d_maxn2, &h->d_sub, &h->d_gx, &h->d_rows16, &h->d_f16st, &h->d_gx16, &h->d_half_stats,
+                      &h->d_rows8, &h->d_q8sx, &h->d_q8e})
         free_dev(*b);
     for (Lane& l : h->lanes)
         for (DevBuf* b : {&l.d_q, &l.d_keys0, &l.d_keys1, &l.d_sched, &l.d_flist, &l.d_fscratch, &l.d_cert}) free_dev(*b);
@@ -217,6 +219,10 @@ int mlv_index_set_tuning(mlv_index_t h, const char* key, int value) {
     else if (k == "scan_half") {
         h->tune_scan_half = value;
         h->half_skip = h->half_backoff = 0;
+        h->q8_skip = h->q8_backoff = 0;
+    } else if (k == "scan_q8") {
+        h->tune_scan_q8 = value;
+        h->q8_skip = h->q8_backoff = 0;
     } else if (k == "gemm_predict") {
         h->tune_gemm_predict = value;
         h->gemm_predict_skip = h->gemm_predict_backoff = 0;
@@ -404,6 +410,7 @@ int mlv_index_compact(mlv_index_t h, int64_t* old_to_new, uint64_t* new_rows) {
     h->n_deleted = 0;
     h->norms_valid = 0;
     h->f16_valid = 0;
+    h->q8_valid = 0;
     h->epoch++;
     h->compact_gen++;
     CK(h, cudaMemsetAsync(h->d_live, 0, h->live_words * 4, h->stream));
@@ -429,6 +436,7 @@ int mlv_index_clear(mlv_index_t h) {
     h->n_deleted = 0;
     h->norms_valid = 0;
     h->f16_valid = 0;
+    h->q8_valid = 0;
     h->epoch++;
     h->compact_gen++;
     drop_columns(h);
@@ -1160,7 +1168,8 @@ int mlv_index_info(mlv_index_t h, mlv_index_info_t* info) {
     info->row_base = h->row_base;
     size_t b = (size_t)h->capacity * h->ld * 4 + (size_t)h->live_words * 4;
     for (const DevBuf* d : {&h->d_qraw, &h->d_filter, &h->d_outd, &h->d_outr, &h->d_outc, &h->d_misc, &h->d_range, &h->d_norms,
-                            &h->d_gq, &h->d_cand, &h->d_maxn2, &h->d_rows16, &h->d_gx, &h->d_gx16})
+                            &h->d_gq, &h->d_cand, &h->d_maxn2, &h->d_rows16, &h->d_gx, &h->d_gx16,
+                            &h->d_rows8, &h->d_q8sx})
         b += d->bytes;
     for (const Lane& l : h->lanes)
         for (const DevBuf* d : {&l.d_q, &l.d_keys0, &l.d_keys1, &l.d_sched, &l.d_flist, &l.d_fscratch}) b += d->bytes;
@@ -1246,12 +1255,15 @@ int mlv_index_gemm_stats(mlv_index_t h, mlv_gemm_stats_t* out) {
     out->half_queries = h->gemm_half_queries;
     out->mispredicted_queries = h->gemm_mispredicted_queries;
     out->half_scan_queries = out->half_scan_uncertified = 0;
-    if (h->d_half_stats.p) {   // counters the shadow-scan kernels keep on the device
-        uint32_t hs[2] = {0, 0};
+    out->q8_scan_queries = out->q8_scan_uncertified = 0;
+    if (h->d_half_stats.p) {   // counters the shadow-scan kernels keep on the device: {fp16 q, uncertified, int8 q, uncertified}
+        uint32_t hs[4] = {0, 0, 0, 0};
         CK(h, cudaDeviceSynchronize());
-        CK(h, cudaMemcpy(hs, h->d_half_stats.p, 8, cudaMemcpyDeviceToHost));
-        out->half_scan_queries = hs[0];
-        out->half_scan_uncertified = hs[1];
+        CK(h, cudaMemcpy(hs, h->d_half_stats.p, 16, cudaMemcpyDeviceToHost));
+        out->half_scan_queries = (uint64_t)hs[0] + hs[2];
+        out->half_scan_uncertified = (uint64_t)hs[1] + hs[3];
+        out->q8_scan_queries = hs[2];
+        out->q8_scan_uncertified = hs[3];
     }
     out->gathered_searches = h->gemm_gathered_searches;
     out->rounds = h->gemm_rounds;
@@ -1336,6 +1348,49 @@ int mlv_index_debug_half_scan(mlv_index_t h, const float* query, float* out_appr
     out_info->scale = out[h->rows + 2];
     out_info->overflow = f16st[2];
     out_info->consumers = c.R == 16 ? 2u : 1u;   // rows too long for two 16-row stages take the FMA consumers
+    return MLV_OK;
+}
+
+int mlv_index_debug_q8_scan(mlv_index_t h, const float* query, float* out_approx, mlv_q8_scan_debug_t* out_info) {
+    if (!h) return MLV_E_INVALID;
+    if (!query || !out_approx || !out_info) return fail(h, MLV_E_INVALID, "bad argument");
+    if (h->rows == 0 || h->rows > SELECT_MAX_P) return fail(h, MLV_E_UNSUPPORTED, "debug_q8_scan needs 1..8192 rows");
+    DeviceGuard g(h->device);
+    cudaStream_t st = h->stream;
+    Lane* ln = lane_for(h, st);
+    int rc;
+    if ((rc = ensure_dev(h, h->d_qraw, (size_t)h->dim * 4)) != MLV_OK) return rc;
+    CK(h, cudaMemcpyAsync(h->d_qraw.p, query, (size_t)h->dim * 4, cudaMemcpyHostToDevice, st));
+    if ((rc = prep_queries(h, (const float*)h->d_qraw.p, 1, st)) != MLV_OK) return rc;
+    bool usable = false;
+    if ((rc = ensure_shadow(h, st, &usable, true)) != MLV_OK) return rc;
+    if (!usable) return fail(h, MLV_E_NOMEM, "no room for the int8 shadow");
+    ScanCfg c;
+    if ((rc = choose_cfg(h, 1, 1, true, &c, false, SHADOW_Q8)) != MLV_OK) return rc;
+    ScanParams p = q8_params(h, c, FilterPlan{}, ln, 1);
+    p.sched = nullptr;
+    p.queries = reinterpret_cast<const float4*>(ln->d_q.p);
+    p.nq_valid = 1;
+    // [rows] approximate distances (+inf where the kernel stores nothing) | |q|^2, t, delta
+    const size_t n_out = (size_t)h->rows + 3;
+    if ((rc = ensure_dev(h, h->d_outd, n_out * 4)) != MLV_OK) return rc;
+    std::vector<float> out(n_out, std::numeric_limits<float>::infinity());
+    CK(h, cudaMemcpyAsync(h->d_outd.p, out.data(), n_out * 4, cudaMemcpyHostToDevice, st));
+    p.out_dists = (float*)h->d_outd.p;
+    CK(h, h->metric == MLV_L2 ? launch_smem<scan_kernel_q8_debug<METRIC_L2>>(c, st, p) : launch_smem<scan_kernel_q8_debug<METRIC_IP>>(c, st, p));
+    h->launches++;
+    uint32_t e_bits = 0, maxn2 = 0;
+    CK(h, cudaMemcpyAsync(out.data(), h->d_outd.p, n_out * 4, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaMemcpyAsync(&e_bits, h->d_q8e.p, 4, cudaMemcpyDeviceToHost, st));
+    if (h->metric != MLV_COSINE) CK(h, cudaMemcpyAsync(&maxn2, h->d_maxn2.p, 4, cudaMemcpyDeviceToHost, st));
+    CK(h, cudaStreamSynchronize(st));
+    memcpy(out_approx, out.data(), (size_t)h->rows * 4);
+    out_info->q_norm2 = out[h->rows];
+    out_info->q_scale = out[h->rows + 1];
+    out_info->delta = out[h->rows + 2];
+    memcpy(&out_info->max_norm2, &maxn2, 4);
+    memcpy(&out_info->e_max, &e_bits, 4);
+    out_info->ld8 = q8_ld(h);
     return MLV_OK;
 }
 

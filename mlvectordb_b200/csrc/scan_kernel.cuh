@@ -47,7 +47,28 @@ __host__ __device__ inline int f16_scale_exp(float m) {
     return s < -100 ? -100 : (s > 100 ? 100 : s);
 }
 
+// Int8 shadow (scan_kernel_q8): a row is x = s_x x^ + e with int8 digits x^, one scale per row and |e|_2 <= e_x <= E (every
+// e_x rounded up, E their maximum); the query is q = t (h + l / 254) + r with int8 digits h, l.  The consumers compute
+// a = s_x t (D_h + D_l / 254) from the exact int32 sums D_h = x^.h and D_l = x^.l, and
+//   x.q - s_x t (D_h + D_l / 254) = e.q + s_x x^.r,   |e.q| <= E |q|,   |s_x x^.r| <= (|x|max + E) |r|   (Cauchy-Schwarz).
+// fp32 rounding: converting the sums, the product with fl(1/254), their sum and the two scale products are <= 12 roundings
+// of terms each at most A tq (A = |x|max + E, tq = t (|h| + |l| / 254)): <= 2^-20 A tq.  The exact side is the fp32 scan's
+// own sum, off by <= d 2^-23 |x||q|, and 1 - dot on either side adds <= 2^-24 (1 + |dot|); all of it is below
+// (d + 64) 2^-22 A (|q| + tq) + 2^-22.  l2: a = |x|^2 + |q|^2 - 2 dot with fp32 norms (each off by <= d 2^-23 of itself)
+// against the fp32 sum of (x - q)^2 (off by <= (d + 2) 2^-23 (|x| + |q|)^2): twice the dot terms plus
+// (d + 64) 2^-21 (A + |q| + tq)^2.  Returns the bound on |a - exact| for every row (absolute, not relative to a scale).
+__host__ __device__ inline float q8_delta(bool l2, uint32_t d, float xmax, float E, float qn, float rn, float tq) {
+    const float A = xmax + E;
+    const float dot = E * qn + A * rn;
+    const float eps = (float)(d + 64) * 2.384185791015625e-7f;
+    if (!l2) return dot + eps * A * (qn + tq) + 2.384185791015625e-7f;
+    const float w = A + qn + tq;
+    return 2.0f * dot + 2.0f * eps * w * w;
+}
+
 constexpr uint32_t SCAN_FUSED_MAX_KEYS = 8192;  // keys the last CTA folds (gridDim.x * k): k <= 55 on 148 SMs
+// ... the int8 shadow scan's k' = 64 on 148 SMs (9472 keys): 128 KB of candidate slots in its idle ring
+constexpr uint32_t SCAN_FUSED_MAX_KEYS_Q8 = 16384;
 
 struct ScanParams {
     const float4* rows;     // [n_rows, ld4]
@@ -113,7 +134,7 @@ struct ScanParams {
     // fence + flag cost 4 us of a 27 us launch on a 10k-row namespace).
     uint4* tagged_out;
     unsigned int tag;
-    // ---- shadow scan (HALF instantiations: one query, k' = k <= 32 candidates, fused tail) -------------------------
+    // ---- shadow scan (HALF instantiations: one query, k' = k <= 64 candidates, fused tail) -------------------------
     // rows / ld4 / stage_f4 describe the fp16 SHADOW of the matrix (halves of row * 2^s, ld4 = 16-byte units per row):
     // the pass reads half the bytes and selects k' candidates by approximate distance; the last CTA re-scores them from
     // the fp32 matrix in the scan's own arithmetic, keeps the best k_out and certifies the answer exactly like the
@@ -131,8 +152,14 @@ struct ScanParams {
     // fallback is decided on the device, no host synchronisation
     uint32_t* cert;
     const uint32_t* run_if;
-    uint32_t* half_stats;            // device counters {shadow-scan queries, not certified}
-    volatile uint32_t* half_stats_host;  // mapped pinned mirror {queries, not certified, overflow flag} (plain stores)
+    // device counters {fp16 queries, not certified, int8 queries, not certified}
+    uint32_t* half_stats;
+    // mapped pinned mirror {fp16 queries, not certified, overflow flag, -, int8 queries, not certified} (plain stores)
+    volatile uint32_t* half_stats_host;
+    // ---- int8 shadow (HALF = 3, scan_kernel_q8): rows / ld4 / stage_f4 describe int8 digits (ld4 = 16-byte units per row),
+    // k' = k <= 64 candidates; the error bound is q8_delta (above), computed per query in the kernel
+    const float* q8_scale;           // s_x per row
+    const uint32_t* q8_e_bits;       // E = max e_x (float bits)
 };
 
 constexpr uint32_t SCAN_INLINE_MAX_DIM = 2048;   // floats of a query carried in the kernel parameters (8 KB)
@@ -261,6 +288,13 @@ __device__ __forceinline__ uint32_t sorted_count_below(const uint64_t* list, uin
     return lo;
 }
 
+// D += A B: A 16 x 32 int8 (row-major fragment a0..a3), B 32 x 8 int8 (b0, b1), int32 accumulators (exact)
+__device__ __forceinline__ void mma_m16n8k32_s8(int (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
+    asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.s8.s8.s32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
+                 : "+r"(c[0]), "+r"(c[1]), "+r"(c[2]), "+r"(c[3])
+                 : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
+}
+
 // D += A B: A 16 x 16 halves (row-major fragment a0..a3), B 16 x 8 halves (b0, b1), fp32 accumulators
 __device__ __forceinline__ void mma_m16n8k16_f16(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0,
                                                  uint32_t b1) {
@@ -274,14 +308,18 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
     constexpr int V = R * NQ;
     static_assert(V <= 32 && (V & (V - 1)) == 0, "R*NQ must be a power of two <= 32");
     // HALF: 0 = the fp32 rows; 1 = the fp16 shadow, FMA consumers; 2 = the fp16 shadow, tensor-core consumers
-    // (mma.sync m16n8k16 on 16 rows x 64 halves per step, the query as halves too; rows of a multiple of 64 halves)
+    // (mma.sync m16n8k16 on 16 rows x 64 halves per step, the query as halves too; rows of a multiple of 64 halves);
+    // 3 = the int8 shadow, tensor-core consumers (mma.sync m16n8k32 s8 on 16 rows x 128 bytes per step, the query as two
+    // int8 digits; rows of a multiple of 128 bytes)
     static_assert(!HALF || (NQ == 1 && !INLINE), "the shadow scan takes one prepared query");
     // DEBUG (scan_kernel_half_debug): the shadow range instantiation's set-up and consumers, but every live row's
     // approximate distance is stored to out_dists[row] instead of being tested, then {|q|^2, 2^-s 2^-t, scale} to
     // out_dists[n_rows ..]; static tile schedule (sched == nullptr), no tail
     static_assert(!DEBUG || (HALF && RANGE), "the debug view is of the shadow range scan");
-    static_assert(HALF != 2 || R == 16, "the tensor-core consumers score 16 rows per step");
-    constexpr bool HMMA = HALF == 2;
+    static_assert(HALF < 2 || R == 16, "the tensor-core consumers score 16 rows per step");
+    constexpr bool Q8 = HALF == 3;
+    static_assert(!Q8 || !RANGE || DEBUG, "the int8 shadow takes single kNN queries");
+    constexpr bool HMMA = HALF >= 2;   // tensor-core consumers: fp16 or int8
     extern __shared__ __align__(128) unsigned char smem[];
     // fallback launch behind a shadow scan: nothing to do when that one certified its answer
     if (NQ == 1 && p.run_if && *reinterpret_cast<const volatile uint32_t*>(p.run_if) == 0) return;   // (single queries only)
@@ -301,17 +339,20 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
     float4* qs = ring + (size_t)S * p.stage_f4;                                   // [NQ][ld4]
     const uint32_t lcap = p.list_cap;             // slots per (warp, query) list
     const bool buffered = lcap > k;               // append buffer + compaction instead of replace-max
-    const uint32_t ldq4 = HALF ? 2 * ld4 : ld4;   // float4 per query in shared memory (HALF: ld4 counts 8-half units)
-    // HMMA: the query once more as halves of q * 2^t ([ld4] 16-byte units), behind the fp32 copy the re-rank reads
+    // float4 per query in shared memory (HALF: ld4 counts 8-half units, Q8: 16-byte units)
+    const uint32_t ldq4 = Q8 ? 4 * ld4 : (HALF ? 2 * ld4 : ld4);
+    // HMMA: the query once more as halves of q * 2^t ([ld4] 16-byte units), behind the fp32 copy the re-rank reads;
+    // Q8: its int8 digits h | l ([ld4] 16-byte units each)
     const unsigned char* q16 = reinterpret_cast<const unsigned char*>(qs + (size_t)NQ * ldq4);
-    uint64_t* lists = reinterpret_cast<uint64_t*>(qs + (size_t)NQ * ldq4 + (HMMA ? ld4 : 0));   // [CW][NQ][lcap]
+    uint64_t* lists = reinterpret_cast<uint64_t*>(qs + (size_t)NQ * ldq4 + (Q8 ? 2 * ld4 : (HMMA ? ld4 : 0)));   // [CW][NQ][lcap]
     uint64_t* full = lists + (RANGE ? 0 : (size_t)CW * NQ * lcap);                // [S]
     uint64_t* empty = full + S;                                                   // [S]
     StageMeta* meta = reinterpret_cast<StageMeta*>(empty + S);                    // [S]
 
     float half_qn = 0.f;                                                           // HALF: |q|^2
     float half_margin = 0.f;                                                       // HALF range mode: candidate margin
-    float half_us = HALF ? __uint_as_float(__ldg(p.half_state)) : 1.0f;            // HALF: 2^-s of the shadow (x 2^-t of the query)
+    float half_us = (HALF && !Q8) ? __uint_as_float(__ldg(p.half_state)) : 1.0f;   // HALF: 2^-s of the shadow (x 2^-t of the query); Q8: t
+    float q8_del = 0.f;                                                            // Q8: the query's q8_delta
     if (tid == 0) {
         for (uint32_t s = 0; s < S; s++) {
             mbar_init(&full[s], 1);
@@ -342,7 +383,7 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
         }
     } else if (HALF) {
         // the fp32 prepared query, zero padded to the shadow's row length; |q|^2 for the l2 form and the certificate
-        __shared__ float s_qn_init, s_q_unscale;
+        __shared__ float s_qn_init, s_q_unscale, s_q8[3];
         for (uint32_t i = tid; i < ldq4; i += blockDim.x)
             qs[i] = i < p.ld4_exact ? p.queries[i] : make_float4(0.f, 0.f, 0.f, 0.f);
         __syncthreads();
@@ -358,7 +399,54 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
 #pragma unroll
             for (int off = 16; off >= 1; off >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, off);
             if (lane == 0) s_qn_init = acc;
-            if (HMMA) {
+            if (Q8) {
+                // q = t (h + l / 254) + r: two int8 digits per element, t = max |q| / 127; zero padding stays zero
+                float m = 0.f;
+                for (uint32_t j = lane; j < ldq4; j += 32) {
+                    const float4 v = qs[j];
+                    m = fmaxf(m, fmaxf(fmaxf(fabsf(v.x), fabsf(v.y)), fmaxf(fabsf(v.z), fabsf(v.w))));
+                }
+#pragma unroll
+                for (int off = 16; off >= 1; off >>= 1) m = fmaxf(m, __shfl_xor_sync(0xffffffffu, m, off));
+                const float t = m / 127.0f, inv = m > 0.f ? 127.0f / m : 0.f, tl = t * (1.0f / 254.0f);
+                uint32_t* dh = reinterpret_cast<uint32_t*>(const_cast<unsigned char*>(q16));
+                uint32_t* dl = dh + ld4 * 4;
+                float rr = 0.f, hh = 0.f, ll = 0.f;
+                for (uint32_t j = lane; j < ldq4; j += 32) {
+                    const float4 v4 = qs[j];
+                    const float v[4] = {v4.x, v4.y, v4.z, v4.w};
+                    uint32_t ph = 0, pl = 0;
+#pragma unroll
+                    for (int i = 0; i < 4; i++) {
+                        const float h = fminf(fmaxf(rintf(v[i] * inv), -127.f), 127.f);
+                        const float r1 = fmaf(-t, h, v[i]);
+                        const float l = fminf(fmaxf(rintf(r1 * inv * 254.0f), -127.f), 127.f);
+                        const float r = fmaf(-tl, l, r1);
+                        rr = fmaf(r, r, rr);
+                        hh = fmaf(h, h, hh);
+                        ll = fmaf(l, l, ll);
+                        ph |= ((uint32_t)(int32_t)h & 0xffu) << (8 * i);
+                        pl |= ((uint32_t)(int32_t)l & 0xffu) << (8 * i);
+                    }
+                    dh[j] = ph;
+                    dl[j] = pl;
+                }
+#pragma unroll
+                for (int off = 16; off >= 1; off >>= 1) {
+                    rr += __shfl_xor_sync(0xffffffffu, rr, off);
+                    hh += __shfl_xor_sync(0xffffffffu, hh, off);
+                    ll += __shfl_xor_sync(0xffffffffu, ll, off);
+                }
+                if (lane == 0) {
+                    // |r| rounded up: the two fmas per element and fl(t / 254) leave <= 2^-22 t each, the sum of squares
+                    // is off by <= d 2^-23 of itself
+                    const float d = (float)(ldq4 * 4);
+                    s_q8[0] = t;
+                    s_q8[1] = sqrtf(rr) * (1.0f + d * 1.1920928955078125e-7f) + t * sqrtf(d) * 2.384185791015625e-7f;
+                    s_q8[2] = t * (sqrtf(hh) + sqrtf(ll) * (1.0f / 254.0f)) * 1.0001f;
+                }
+            }
+            if (HMMA && !Q8) {
                 // halves of q * 2^t, t from the largest component (split_queries_f16_kernel's rule); zero padding stays zero
                 float m = 0.f;
                 for (uint32_t j = lane; j < p.ld4_exact; j += 32) {
@@ -380,8 +468,17 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
         }
         __syncthreads();
         half_qn = s_qn_init;
-        if (HMMA) half_us *= s_q_unscale;
-        if (RANGE) {
+        if (HMMA && !Q8) half_us *= s_q_unscale;
+        if (Q8) {
+            half_us = s_q8[0];
+            const float xmax = p.cosine ? 1.0f : sqrtf(__uint_as_float(*p.max_norm2_bits));
+            q8_del = q8_delta(METRIC == METRIC_L2, p.ld4_exact * 4, xmax, __uint_as_float(*p.q8_e_bits), sqrtf(half_qn), s_q8[1], s_q8[2]);
+            if (DEBUG && blockIdx.x == 0 && tid == 0) {
+                p.out_dists[p.n_rows] = half_qn;
+                p.out_dists[p.n_rows + 1] = half_us;
+                p.out_dists[p.n_rows + 2] = q8_del;
+            }
+        } else if (RANGE) {
             // shadow range scan: a row is a CANDIDATE when its approximate distance is within the fp16 error bound of the
             // radius; candidates are re-scored from the fp32 matrix on the spot and tested exactly, so the hit list is the
             // fp32 scan's by construction -- no certificate, no second launch.  An overflowed shadow makes every row a
@@ -551,7 +648,42 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
             float xn = 0.f;
             if (HALF && METRIC == METRIC_L2) xn = __ldg(p.row_norms + (p.gather ? row : pos));   // own slot's row; in flight during the dot products
             float s_mma = 0.f;
-            if constexpr (HMMA) {
+            if constexpr (Q8) {
+                // Int8 consumers: the fp16 consumers' access pattern below, with 32 bytes of k per instruction.  B columns
+                // n with bit 1 clear take the query's high digit h, the others its low digit l, so one MMA yields both sums
+                // for a row: D_h in column (row parity), D_l in column (row parity) + 2 -- lanes t = 0 and t = 1 of the row
+                // group, which trade one value so that t == 0 holds both sums of row g and t == 1 both of row g + 8.
+                const float xs = __ldg(p.q8_scale + pos);
+                const int g = lane >> 2, t = lane & 3;
+                const uint32_t rowbytes = ld4 * 16;
+                const unsigned char* r0 = reinterpret_cast<const unsigned char*>(tile) + (size_t)(base + g) * rowbytes;
+                const unsigned char* r1 = r0 + 8 * (size_t)rowbytes;
+                const unsigned char* qd = q16 + ((g & 2) ? rowbytes : 0u);
+                int c[4] = {0, 0, 0, 0}, d[4] = {0, 0, 0, 0};
+                const uint32_t o0 = (uint32_t)(t + 4 * (g & 1)) * 16, o1 = (uint32_t)(t + 4 * ((g & 1) ^ 1)) * 16;
+                for (uint32_t ch = 0; ch < rowbytes; ch += 128) {
+                    {
+                        const uint4 xa = *reinterpret_cast<const uint4*>(r0 + ch + o0);
+                        const uint4 xb = *reinterpret_cast<const uint4*>(r1 + ch + o0);
+                        const uint4 qv = *reinterpret_cast<const uint4*>(qd + ch + o0);
+                        mma_m16n8k32_s8(c, xa.x, xb.x, xa.y, xb.y, qv.x, qv.y);
+                        mma_m16n8k32_s8(d, xa.z, xb.z, xa.w, xb.w, qv.z, qv.w);
+                    }
+                    {
+                        const uint4 xa = *reinterpret_cast<const uint4*>(r0 + ch + o1);
+                        const uint4 xb = *reinterpret_cast<const uint4*>(r1 + ch + o1);
+                        const uint4 qv = *reinterpret_cast<const uint4*>(qd + ch + o1);
+                        mma_m16n8k32_s8(c, xa.x, xb.x, xa.y, xb.y, qv.x, qv.y);
+                        mma_m16n8k32_s8(d, xa.z, xb.z, xa.w, xb.w, qv.z, qv.w);
+                    }
+                }
+                // lane (g, t) holds C[g][2t + j] (j = 0, 1) and C[g + 8][2t + j]; the row parity picks j
+                const int par = g & 1;
+                const int lo_g = par ? c[1] + d[1] : c[0] + d[0], lo_g8 = par ? c[3] + d[3] : c[2] + d[2];
+                const int got = __shfl_xor_sync(0xffffffffu, t == 0 ? lo_g8 : lo_g, 1);
+                const int dh = t == 0 ? lo_g : got, dl = t == 0 ? got : lo_g8;
+                s_mma = xs * ((float)dh + (float)dl * (1.0f / 254.0f));
+            } else if constexpr (HMMA) {
                 // Tensor-core consumers.  The dot product does not care in which order k is walked, as long as rows and
                 // query agree: lane (g, t) feeds the fragment slots (row g / g + 8, k 2t.. and 2t + 8..) with the 16 bytes
                 // at offset 16 (t + 4 ((g & 1) ^ step)) of the rows' current 128-byte chunk, and the B fragment (column n
@@ -930,10 +1062,10 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
         uint32_t kf = k;
         uint32_t my_uncert = 0;   // HALF: bit qi = query qi is not certified on this rank (same in every thread)
         if (HALF) {
-            // ---- exact re-rank of the k' <= 32 candidates + certificate (see ScanParams) ----
+            // ---- exact re-rank of the k' <= 64 candidates + certificate (see ScanParams) ----
             __shared__ uint32_t s_uncert;
-            uint64_t* ex = top + (size_t)p.nq_valid * k;        // [nq][32] exact keys, unsorted
-            uint64_t* fx = ex + (size_t)p.nq_valid * 32;        // [nq][k_out] exact keys, ascending
+            uint64_t* ex = top + (size_t)p.nq_valid * k;        // [nq][64] exact keys, unsorted
+            uint64_t* fx = ex + (size_t)p.nq_valid * 64;        // [nq][k_out] exact keys, ascending
             if (tid == 0) s_uncert = 0;
             // four candidates per warp at a time: their rows are four independent HBM round trips (a candidate at a time
             // cost ~1.5 us each, 8 per warp); per candidate the scan's own arithmetic -- lane l sums float4 columns l,
@@ -960,28 +1092,32 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
                     for (int off = 16; off >= 1; off >>= 1) a += __shfl_xor_sync(0xffffffffu, a, off);
                     if (lane == 0 && e0 + u < p.nq_valid * k) {
                         const uint32_t qi = (e0 + u) / k, i = (e0 + u) - qi * k;
-                        ex[qi * 32 + i] = keys[u] != KEY_SENTINEL ? make_key((METRIC == METRIC_IP) ? 1.0f - a : a, key_row(keys[u])) : KEY_SENTINEL;
+                        ex[qi * 64 + i] = keys[u] != KEY_SENTINEL ? make_key((METRIC == METRIC_IP) ? 1.0f - a : a, key_row(keys[u])) : KEY_SENTINEL;
                     }
                 }
             }
             named_bar_sync(1, CW * 32);
             if ((uint32_t)warp < p.nq_valid) {
                 const uint32_t qi = (uint32_t)warp;
-                uint64_t v = (uint32_t)lane < k ? ex[qi * 32 + lane] : KEY_SENTINEL;
-                v = warp_bitonic_sort_u64(v, lane);
-                if ((uint32_t)lane < p.k_out) fx[qi * p.k_out + lane] = v;
+                uint64_t* xs = ex + qi * 64;
+                warp_sort_list(xs, k, 64, lane);
+                if ((uint32_t)lane < p.k_out) fx[qi * p.k_out + lane] = xs[lane];
                 const uint64_t last = top[qi * k + k - 1];                 // k'-th approximate key: sentinel = every row is a candidate
-                const uint64_t ek = shfl_u64(v, (int)p.k_out - 1);         // exact k-th best among the candidates
+                const uint64_t ek = xs[p.k_out - 1];                       // exact k-th best among the candidates
                 bool certified = true;
                 if (last != KEY_SENTINEL) {
-                    float scale = 1.0f;
-                    if (!p.cosine) {
-                        const float xmax = sqrtf(__uint_as_float(*p.max_norm2_bits)), qsn = sqrtf(half_qn);
-                        scale = (METRIC == METRIC_L2) ? (xmax + qsn) * (xmax + qsn) : xmax * qsn;
+                    float delta = q8_del;
+                    if (!Q8) {
+                        float scale = 1.0f;
+                        if (!p.cosine) {
+                            const float xmax = sqrtf(__uint_as_float(*p.max_norm2_bits)), qsn = sqrtf(half_qn);
+                            scale = (METRIC == METRIC_L2) ? (xmax + qsn) * (xmax + qsn) : xmax * qsn;
+                        }
+                        delta = p.delta_rel * scale;
                     }
-                    certified = (key_dist(last) - p.delta_rel * scale > key_dist(ek));   // false for NaN
+                    certified = (key_dist(last) - delta > key_dist(ek));   // false for NaN
                 }
-                if (__ldg(p.half_state + 2)) certified = false;   // the shadow overflowed fp16: nothing it selected can be trusted
+                if (!Q8 && __ldg(p.half_state + 2)) certified = false;   // the shadow overflowed fp16: nothing it selected can be trusted
                 if (lane == 0 && !certified) atomicOr(&s_uncert, 1u << qi);
             }
             named_bar_sync(1, CW * 32);
@@ -1029,12 +1165,13 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
         if (NQ == 1 && p.cert && tid == 0) {
             *p.cert = any_uncert ? 1u : 0u;
             if (HALF) {
-                const uint32_t a = atomicAdd(p.half_stats, p.nq_valid) + p.nq_valid;
-                const uint32_t b = atomicAdd(p.half_stats + 1, (uint32_t)__popc(my_uncert)) + (uint32_t)__popc(my_uncert);
+                uint32_t* cnt = p.half_stats + (Q8 ? 2 : 0);
+                const uint32_t a = atomicAdd(cnt, p.nq_valid) + p.nq_valid;
+                const uint32_t b = atomicAdd(cnt + 1, (uint32_t)__popc(my_uncert)) + (uint32_t)__popc(my_uncert);
                 if (p.half_stats_host) {
-                    p.half_stats_host[0] = a;
-                    p.half_stats_host[1] = b;
-                    p.half_stats_host[2] = __ldg(p.half_state + 2);
+                    p.half_stats_host[Q8 ? 4 : 0] = a;
+                    p.half_stats_host[Q8 ? 5 : 1] = b;
+                    if (!Q8) p.half_stats_host[2] = __ldg(p.half_state + 2);
                 }
             }
         }
@@ -1077,6 +1214,11 @@ template <int METRIC, bool RANGE = false>
 __global__ void __launch_bounds__(256, 1) scan_kernel_half_mma(const ScanParams p) {   // <= 7 consumer warps + 1 producer
     scan_body<METRIC, 1, 16, RANGE, false, 2>(p, nullptr);
 }
+// one query over the int8 shadow (rows of a multiple of 128 bytes), int8 tensor-core consumers, k' <= 64
+template <int METRIC>
+__global__ void __launch_bounds__(256, 1) scan_kernel_q8(const ScanParams p) {   // <= 7 consumer warps + 1 producer
+    scan_body<METRIC, 1, 16, false, false, 3>(p, nullptr);
+}
 // tests only (mlv_index_debug_half_scan): the approximate distance of every live row, from the consumers above
 template <int METRIC, int R>
 __global__ void __launch_bounds__(scan_max_threads<4>(), 1) scan_kernel_half_debug(const ScanParams p) {
@@ -1085,6 +1227,11 @@ __global__ void __launch_bounds__(scan_max_threads<4>(), 1) scan_kernel_half_deb
 template <int METRIC>
 __global__ void __launch_bounds__(256, 1) scan_kernel_half_mma_debug(const ScanParams p) {
     scan_body<METRIC, 1, 16, true, false, 2, true>(p, nullptr);
+}
+// tests only (mlv_index_debug_q8_scan): the int8 consumers' approximate distance of every live row, then {|q|^2, t, delta}
+template <int METRIC>
+__global__ void __launch_bounds__(256, 1) scan_kernel_q8_debug(const ScanParams p) {
+    scan_body<METRIC, 1, 16, true, false, 3, true>(p, nullptr);
 }
 // one query whose raw values travel in the launch parameters (batch-1 latency path)
 template <int METRIC, int R, bool RANGE>

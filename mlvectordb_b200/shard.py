@@ -407,6 +407,16 @@ class DeviceShard:
                                                      C.byref(info)))
         return out, {f: getattr(info, f) for f, _ in info._fields_}
 
+    def debug_q8_scan(self, query: np.ndarray) -> Tuple[np.ndarray, dict]:
+        """Approximate distances [rows] the int8 shadow scan's consumers compute for one query (+inf for tombstoned rows)
+        and what its certificate is computed from (``mlv_q8_scan_debug_t`` as a dict; tests only)."""
+        q = np.ascontiguousarray(query, dtype=np.float32).reshape(self.dim)
+        out = np.empty(self.rows, dtype=np.float32)
+        info = _capi.Q8ScanDebug()
+        self._ck(self._lib.mlv_index_debug_q8_scan(self._h, q.ctypes.data_as(C.c_void_p), out.ctypes.data_as(C.c_void_p),
+                                                   C.byref(info)))
+        return out, {f: getattr(info, f) for f, _ in info._fields_}
+
     def kernel_launches(self) -> int:
         n = C.c_uint64()
         self._ck(self._lib.mlv_index_kernel_launches(self._h, C.byref(n)))
