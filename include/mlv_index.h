@@ -254,6 +254,34 @@ int mlv_index_get_column(mlv_index_t h, uint32_t column, uint64_t first_row, uin
 int mlv_filter_create_where(mlv_index_t h, const mlv_predicate_t *preds, uint32_t n_preds, mlv_filter_t *out);
 
 /*
+ * Grouped search: the k nearest GROUPS of `column`, one best row per group (group-by search: the k nearest documents
+ * rather than the k nearest chunks).  A row's group is its code in `column`.  Per query q:
+ *   1. L = the rows that are live, pass the filter and hold a value other than MLV_COLUMN_MISSING in `column`, ordered
+ *      as mlv_index_search orders results: by (d, row), d the fp32 scan's arithmetic bit for bit;
+ *   2. walk L and keep the first row of every group not seen yet; stop after k rows;
+ *   3. return them ascending: out_dists / out_rows [nq, k] as in mlv_index_search, out_groups [nq, k] their codes,
+ *      out_counts [nq] = min(k, distinct groups in L).  Padding: +inf / -1 / MLV_COLUMN_MISSING.
+ * So a group is reported with its best member, ties between equal distances go to the lower row, and when every row is
+ * its own group the answer is mlv_index_search's.  Rows without a value are in no group.
+ * 1 <= k <= MLV_MAX_GROUP_K (k == 0: MLV_E_INVALID; larger: MLV_E_UNSUPPORTED); column >= MLV_MAX_COLUMNS: MLV_E_INVALID.
+ * A column never written holds no groups: every count is 0.  A bound prepared filter, tombstones and the per-call bitmap
+ * apply as in every other search.  The pass is always the fp32 scan -- never a shadow scan, the tensor-core batch path,
+ * the latency path or an attached exchange -- in passes of up to 8 queries, each finished by its last CTA (so
+ * set_tuning "dynamic" and "fused" must be 1: MLV_E_UNSUPPORTED otherwise).  A group's code is read only for rows that
+ * beat the current k-th best, so the pass moves the bytes of a plain search.
+ * Not (yet) offered: shadow scans, the tensor-core batch path, range search by group, more than one row per group,
+ * k > MLV_MAX_GROUP_K.  The host variant blocks until the results are in the host buffers; the device variant is
+ * enqueued on `stream` like mlv_index_search_device.
+ */
+#define MLV_MAX_GROUP_K 32u
+int mlv_index_search_grouped(mlv_index_t h, const float *queries, uint32_t nq, uint32_t k, uint32_t column,
+                             const uint32_t *filter_bitmap, float *out_dists, int64_t *out_rows,
+                             int32_t *out_groups, int32_t *out_counts);
+int mlv_index_search_grouped_device(mlv_index_t h, const float *queries_dev, uint32_t nq, uint32_t k, uint32_t column,
+                                    const uint32_t *filter_bitmap_dev, float *out_dists_dev, int64_t *out_rows_dev,
+                                    int32_t *out_groups_dev, int32_t *out_counts_dev, void *stream);
+
+/*
  * Snapshot support (SURVEY.md section 8f rank 4; the reference has no persistence, README.md:240-241 only):
  * rows exactly as stored (cosine: already normalised), tombstoned ones included, and the tombstone bitmap
  * (bit set = live).  mlv_index_import_rows appends stored-form rows WITHOUT normalising them again, so an
@@ -355,7 +383,8 @@ int mlv_index_scan_time_ms(mlv_index_t h, double *total_ms, uint64_t *launches);
  * 1 = filters always gather; the tensor-core path compacts the passing rows accordingly), "staged_upload"
  * (1 = bulk mlv_index_add through two pinned chunks filled by worker threads, 0 = plain copy), "fast_host" (1 = single-query
  * mlv_index_search takes the one-launch latency path, 0 = always staged), "scan_half" / "scan_half_mma" / "scan_q8" (below), and the
- * tensor-core keys listed at mlv_index_gemm_stats}.  Results never depend on these.
+ * tensor-core keys listed at mlv_index_gemm_stats}.  Results never depend on these, with one exception: a grouped search
+ * (mlv_index_search_grouped) returns MLV_E_UNSUPPORTED while "dynamic" or "fused" is 0.
  *
  * Shadow scan ("scan_half": -1 auto = matrices of 256 MB and more, 0 never, 1 whenever the shape allows).  A SINGLE
  * query with k <= 16 reads an fp16 shadow of the rows -- half the bytes of the HBM-bound pass; the

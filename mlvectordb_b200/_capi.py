@@ -99,6 +99,7 @@ class Predicate(C.Structure):
 
 
 MAX_COLUMNS, MAX_PREDICATES = 16, 8
+MAX_GROUP_K = 32
 COLUMN_MISSING = -(2 ** 31)
 PRED_OPS = {"==": 0, "!=": 1, "<": 2, "<=": 3, ">": 4, ">=": 5, "between": 6}
 
@@ -150,6 +151,10 @@ SIGNATURES = {
     "mlv_index_set_column": (C.c_int, [_h, C.c_uint32, C.c_uint64, C.c_void_p, C.c_uint64]),
     "mlv_index_set_column_device": (C.c_int, [_h, C.c_uint32, C.c_uint64, C.c_void_p, C.c_uint64]),
     "mlv_index_get_column": (C.c_int, [_h, C.c_uint32, C.c_uint64, C.c_uint64, C.c_void_p]),
+    "mlv_index_search_grouped": (C.c_int, [_h, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p,
+                                           C.c_void_p, C.c_void_p, C.c_void_p]),
+    "mlv_index_search_grouped_device": (C.c_int, [_h, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint32, C.c_void_p, C.c_void_p,
+                                                  C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "mlv_format_f32_json": (C.c_int, [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint64, _u64p]),
     "mlv_index_export_rows": (C.c_int, [_h, C.c_uint64, C.c_uint64, C.c_void_p]),
     "mlv_index_export_live": (C.c_int, [_h, C.c_void_p, C.c_uint64]),

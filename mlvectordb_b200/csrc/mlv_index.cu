@@ -912,6 +912,67 @@ int mlv_index_search_exchange(mlv_index_t h, const float* queries, uint32_t nq, 
     return search_host_common(h, queries, nq, k, filter_bitmap, out_dists, out_rows, out_counts, true);
 }
 
+// argument checks both grouped entries share (pointers and nq aside)
+static int grouped_args(mlv_index_t h, uint32_t k, uint32_t column) {
+    if (k == 0 || column >= MLV_MAX_COLUMNS) return fail(h, MLV_E_INVALID, "bad argument");
+    if (k > MLV_MAX_GROUP_K) return fail(h, MLV_E_UNSUPPORTED, "k exceeds MLV_MAX_GROUP_K");
+    if (!h->tune_dynamic || !h->tune_fused)
+        return fail(h, MLV_E_UNSUPPORTED, "grouped search finishes in the fused last-CTA tail: set_tuning \"dynamic\" and \"fused\" must be 1");
+    return MLV_OK;
+}
+
+int mlv_index_search_grouped_device(mlv_index_t h, const float* queries_dev, uint32_t nq, uint32_t k, uint32_t column,
+                                    const uint32_t* filter_bitmap_dev, float* out_dists_dev, int64_t* out_rows_dev,
+                                    int32_t* out_groups_dev, int32_t* out_counts_dev, void* stream) {
+    NvtxRange nvtx_range("mlv_index_search_grouped_device");
+    if (!h || !queries_dev || !out_dists_dev || !out_rows_dev || !out_groups_dev || !out_counts_dev || nq == 0) return fail(h, MLV_E_INVALID, "bad argument");
+    int rc = grouped_args(h, k, column);
+    if (rc != MLV_OK) return rc;
+    DeviceGuard g(h->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    if (h->rows == h->n_deleted || !h->d_cols[column].p) {   // nothing live, or a column never written: no groups
+        fill_empty_kernel<<<32, 256, 0, st>>>(out_dists_dev, out_rows_dev, out_counts_dev, nq, k);
+        fill_i32_kernel<<<32, 256, 0, st>>>(out_groups_dev, (uint64_t)nq * k, COLUMN_MISSING);
+        h->launches += 2;
+        CK(h, cudaGetLastError());
+        return MLV_OK;
+    }
+    if ((rc = prep_queries(h, queries_dev, nq, st)) != MLV_OK) return rc;
+    return search_grouped(h, (const float*)lane_for(h, st)->d_q.p, nq, k, (const int32_t*)h->d_cols[column].p, h->col_rows[column],
+                          filter_bitmap_dev, out_dists_dev, out_rows_dev, out_groups_dev, out_counts_dev, st);
+}
+
+int mlv_index_search_grouped(mlv_index_t h, const float* queries, uint32_t nq, uint32_t k, uint32_t column, const uint32_t* filter_bitmap,
+                             float* out_dists, int64_t* out_rows, int32_t* out_groups, int32_t* out_counts) {
+    NvtxRange nvtx_range("mlv_index_search_grouped");
+    if (!h || !queries || !out_dists || !out_rows || !out_groups || !out_counts || nq == 0) return fail(h, MLV_E_INVALID, "bad argument");
+    int rc = grouped_args(h, k, column);
+    if (rc != MLV_OK) return rc;
+    DeviceGuard g(h->device);
+    const size_t qbytes = (size_t)nq * h->dim * 4;
+    const size_t nk = (size_t)nq * k;
+    const size_t out_bytes = nk * 16 + (size_t)nq * 4;   // rows | dists | groups | counts: one copy brings them back
+    if ((rc = ensure_host(h, h->h_stage, std::max(qbytes, out_bytes))) != MLV_OK) return rc;
+    if ((rc = ensure_dev(h, h->d_qraw, qbytes)) != MLV_OK) return rc;
+    if ((rc = ensure_dev(h, h->d_outr, out_bytes)) != MLV_OK) return rc;
+    char* d = (char*)h->d_outr.p;
+    const uint32_t* filter_dev;
+    if ((rc = upload_filter_bitmap(h, filter_bitmap, &filter_dev)) != MLV_OK) return rc;
+    memcpy(h->h_stage.p, queries, qbytes);
+    CK(h, cudaMemcpyAsync(h->d_qraw.p, h->h_stage.p, qbytes, cudaMemcpyHostToDevice, h->stream));
+    rc = mlv_index_search_grouped_device(h, (const float*)h->d_qraw.p, nq, k, column, filter_dev, (float*)(d + nk * 8), (int64_t*)d,
+                                         (int32_t*)(d + nk * 12), (int32_t*)(d + nk * 16), h->stream);
+    if (rc != MLV_OK) return rc;
+    char* hs = (char*)h->h_stage.p;
+    CK(h, cudaMemcpyAsync(hs, d, out_bytes, cudaMemcpyDeviceToHost, h->stream));
+    CK(h, cudaStreamSynchronize(h->stream));
+    memcpy(out_rows, hs, nk * 8);
+    memcpy(out_dists, hs + nk * 8, nk * 4);
+    memcpy(out_groups, hs + nk * 12, nk * 4);
+    memcpy(out_counts, hs + nk * 16, (size_t)nq * 4);
+    return MLV_OK;
+}
+
 int mlv_index_submit(mlv_index_t h, const float* queries, uint32_t nq, uint32_t k, int exchange, uint32_t* ticket) {
     NvtxRange nvtx_range("mlv_index_submit");
     if (!h || !queries || !ticket || nq == 0 || k == 0) return fail(h, MLV_E_INVALID, "bad argument");

@@ -18,6 +18,7 @@
 //   * at the end the block folds its warps' lists into one list per query and writes
 //     k keys per (query, block); select_kernel.cuh merges the blocks' lists.
 #pragma once
+#include "column_kernels.cuh"
 #include "common.cuh"
 #include "exchange.cuh"
 
@@ -134,6 +135,9 @@ struct ScanParams {
     // fence + flag cost 4 us of a 27 us launch on a 10k-row namespace).
     uint4* tagged_out;
     unsigned int tag;
+    // grouped search (scan_kernel_grouped): rows group_col covers; later rows have no group (this field and the two
+    // unions below fill what would be padding, so every other kernel's parameters keep their offsets)
+    uint32_t group_rows;
     // ---- shadow scan (HALF instantiations: one query, k' = k <= 64 candidates, fused tail) -------------------------
     // rows / ld4 / stage_f4 describe the fp16 SHADOW of the matrix (halves of row * 2^s, ld4 = 16-byte units per row):
     // the pass reads half the bytes and selects k' candidates by approximate distance; the last CTA re-scores them from
@@ -158,8 +162,17 @@ struct ScanParams {
     volatile uint32_t* half_stats_host;
     // ---- int8 shadow (HALF = 3, scan_kernel_q8): rows / ld4 / stage_f4 describe int8 digits (ld4 = 16-byte units per row),
     // k' = k <= 64 candidates; the error bound is q8_delta (above), computed per query in the kernel
-    const float* q8_scale;           // s_x per row
-    const uint32_t* q8_e_bits;       // E = max e_x (float bits)
+    // ---- grouped search (GROUP, scan_kernel_grouped: fp32 rows, kNN, k <= 32) shares the int8 shadow's two slots:
+    // group_col is the int32 column whose code is a row's group (COLUMN_MISSING = no group), out_groups[nq_valid][k]
+    // receives the final rows' codes
+    union {
+        const float* q8_scale;       // s_x per row
+        const int32_t* group_col;
+    };
+    union {
+        const uint32_t* q8_e_bits;   // E = max e_x (float bits)
+        int32_t* out_groups;
+    };
 };
 
 constexpr uint32_t SCAN_INLINE_MAX_DIM = 2048;   // floats of a query carried in the kernel parameters (8 KB)
@@ -288,6 +301,217 @@ __device__ __forceinline__ uint32_t sorted_count_below(const uint64_t* list, uin
     return lo;
 }
 
+// ---- grouped search (GROUP): the k nearest groups of a column, one best row per group --------------------------------
+// A warp list holds at most k entries (key, group) of distinct groups.  Invariant: after any prefix of its rows, it holds
+// the best row of each of the k best groups among those rows, groups ranked by their best key (all groups when fewer).
+// A row of group g with key x below thr (the list's maximum) either improves g's entry (g listed: kept when x is smaller)
+// or, g not listed, replaces the maximum: an earlier row of g lost to k listed groups whose best keys are at most thr, so
+// x < thr is g's best so far and g now ranks above the evicted group.  A row at or above thr cannot be the best row of one
+// of the k best groups.
+// So a row that is the global answer for its group -- its group is among the k best of every subset holding that row --
+// is never lost by the warp that scored it, and the fold and the last-CTA merge only need to de-duplicate by group.
+__device__ __forceinline__ int32_t group_of(const ScanParams& p, uint32_t row) {
+    return row < p.group_rows ? __ldg(p.group_col + row) : COLUMN_MISSING;
+}
+
+// Insert (ckey, cg) into list / groups [k <= 32] (whole warp; lane j owns slot j); oldthr = the list's maximum.  Returns
+// the new maximum.
+__device__ __forceinline__ uint64_t group_list_insert(uint64_t* list, int32_t* groups, uint32_t k, uint64_t ckey, int32_t cg,
+                                                      uint64_t oldthr, int lane) {
+    const bool in = (uint32_t)lane < k;
+    uint64_t v = in ? list[lane] : 0ull;   // lanes without a slot never hold the maximum
+    const unsigned same = __ballot_sync(0xffffffffu, in && groups[lane] == cg);   // (sentinel slots: COLUMN_MISSING)
+    int slot;
+    if (same) {   // at most one: a list never holds a group twice
+        slot = __ffs(same) - 1;
+        if (!(ckey < shfl_u64(v, slot))) return oldthr;
+    } else {
+        slot = __ffs(__ballot_sync(0xffffffffu, in && v == oldthr)) - 1;   // the maximum (a sentinel while not full)
+    }
+    if (lane == slot) {
+        list[slot] = ckey;
+        groups[slot] = cg;
+        v = ckey;
+    }
+    __syncwarp();
+    return warp_max_u64(v);
+}
+
+// 32 (key, group) pairs, one per lane -> ascending by key across the lanes
+__device__ __forceinline__ void warp_bitonic_sort_kg(uint64_t& v, int32_t& g, int lane) {
+#pragma unroll
+    for (int size = 2; size <= 32; size <<= 1) {
+#pragma unroll
+        for (int stride = size >> 1; stride > 0; stride >>= 1) {
+            const uint64_t o = shfl_u64(v, lane ^ stride);
+            const int32_t og = __shfl_sync(0xffffffffu, g, lane ^ stride);
+            const bool keep_min = ((lane & size) == 0) == ((lane & stride) == 0);
+            if (keep_min == (o < v)) {
+                v = o;
+                g = og;
+            }
+        }
+    }
+}
+
+// Threads tid, tid + nthr, ...: first[e] = key[e] is the smallest key of its group among key[0..m) (keys are distinct rows;
+// sentinels are never first); *kept (nullable) counts them.  O(m^2): m is ~k per list on typical data.
+__device__ __forceinline__ void group_firsts(const uint64_t* key, const int32_t* grp, int32_t* first, uint32_t m, uint32_t tid,
+                                             uint32_t nthr, uint32_t* kept) {
+    for (uint32_t e = tid; e < m; e += nthr) {
+        const uint64_t x = key[e];
+        const int32_t g = grp[e];
+        bool f = x != KEY_SENTINEL;
+        for (uint32_t i = 0; i < m && f; i++) f = !(grp[i] == g && key[i] < x);
+        first[e] = f;
+        if (f && kept) atomicAdd(kept, 1u);
+    }
+}
+// number of flagged keys below x
+__device__ __forceinline__ uint32_t group_rank(const uint64_t* key, const int32_t* first, uint32_t m, uint64_t x) {
+    uint32_t r = 0;
+#pragma unroll 4
+    for (uint32_t i = 0; i < m; i++) r += (first[i] != 0) & (key[i] < x);
+    return r;
+}
+
+// Grouped CTA fold (the CW consumer warps; every warp list ascending with its groups): per query, the block's best row of
+// each of its k best groups, ascending and sentinel padded, into out_keys -- the plain fold's survivors-and-rank scheme with
+// survivors de-duplicated by group.  The pool's bound counts only when the pool holds k distinct groups.
+// Scratch: keys sk and groups | flags sg [64 + CW k] each; the pool takes the first 64 slots.
+template <int NQ>
+__device__ void group_fold(const ScanParams& p, const uint64_t* lists, const int32_t* lgroups, uint64_t* sk, int32_t* sg, int CW,
+                           uint32_t tid, uint32_t nthr) {
+    const uint32_t k = p.k, cap = 64u + (uint32_t)CW * k;
+    int32_t* sf = sg + cap;
+    __shared__ uint32_t s_gm, s_gkept;
+    __shared__ unsigned long long s_gT;
+    const uint32_t take = (k + (uint32_t)CW - 1) / (uint32_t)CW;
+    const uint32_t P = min((uint32_t)CW * take, 64u);
+    const uint32_t n_in = (uint32_t)CW * k;
+    for (uint32_t qi = 0; qi < p.nq_valid; qi++) {
+        uint64_t* out = p.out_keys + ((size_t)qi * gridDim.x + blockIdx.x) * k;
+        if (tid < P) {
+            const uint32_t w = tid / take, j = tid - w * take;
+            sk[tid] = lists[((size_t)w * NQ + qi) * k + j];
+            sg[tid] = lgroups[((size_t)w * NQ + qi) * k + j];
+        }
+        if (tid == 0) {
+            s_gm = 0;
+            s_gkept = 0;
+            s_gT = KEY_SENTINEL;
+        }
+        named_bar_sync(1, CW * 32);
+        group_firsts(sk, sg, sf, P, tid, nthr, nullptr);
+        named_bar_sync(1, CW * 32);
+        if (tid < P && sf[tid] && group_rank(sk, sf, P, sk[tid]) == k - 1) s_gT = sk[tid];   // k distinct groups at or below it
+        named_bar_sync(1, CW * 32);
+        const uint64_t T = s_gT;
+        uint64_t* surv = sk + 64;
+        int32_t* survg = sg + 64;
+        int32_t* survf = sf + 64;
+        for (uint32_t e = tid; e < n_in; e += nthr) {
+            const uint32_t w = e / k, j = e - w * k;
+            const uint64_t key = lists[((size_t)w * NQ + qi) * k + j];
+            if (key <= T && key != KEY_SENTINEL) {
+                const uint32_t i = atomicAdd(&s_gm, 1u);
+                surv[i] = key;
+                survg[i] = lgroups[((size_t)w * NQ + qi) * k + j];
+            }
+        }
+        named_bar_sync(1, CW * 32);
+        const uint32_t m = s_gm;
+        group_firsts(surv, survg, survf, m, tid, nthr, &s_gkept);
+        named_bar_sync(1, CW * 32);
+        for (uint32_t e = tid; e < m; e += nthr) {
+            if (!survf[e]) continue;
+            const uint32_t r = group_rank(surv, survf, m, surv[e]);
+            if (r < k) out[r] = surv[e];
+        }
+        for (uint32_t r = s_gkept + tid; r < k; r += nthr) out[r] = KEY_SENTINEL;   // fewer than k groups seen
+        named_bar_sync(1, CW * 32);   // the scratch is reused by the next query
+    }
+}
+
+// Grouped last-CTA merge and outputs (every block list ascending, of distinct groups, sentinel padded).  Bounds on the k-th
+// best group's key: the maximum of a FULL block list (k distinct groups at or below it; a list that is not full ends in a
+// sentinel and bounds nothing), and the k-th smallest head among the heads' first-of-group entries.  Survivors at or below
+// the bound are de-duplicated by group (smallest key) and ranked.  scratch (the whole dynamic shared memory, dead by now):
+// cand [fused_cap] keys | top [nq_valid][k] | groups [fused_cap] | flags [fused_cap].
+template <int NQ>
+__device__ void group_tail(const ScanParams& p, unsigned char* scratch, int CW, uint32_t tid, uint32_t nthr, int lane) {
+    const uint32_t k = p.k, n_lists = gridDim.x, n = n_lists * k;
+    uint64_t* cand = reinterpret_cast<uint64_t*>(scratch);
+    uint64_t* top = cand + p.fused_cap;
+    int32_t* cg = reinterpret_cast<int32_t*>(top + (size_t)p.nq_valid * k);
+    int32_t* cf = cg + p.fused_cap;
+    __shared__ uint32_t s_tm, s_tkept;
+    __shared__ unsigned long long s_tT;
+    for (uint32_t qi = 0; qi < p.nq_valid; qi++) {
+        const uint64_t* keys = p.out_keys + (size_t)qi * n;
+        if (tid == 0) {
+            s_tT = KEY_SENTINEL;
+            s_tm = 0;
+            s_tkept = 0;
+        }
+        named_bar_sync(1, CW * 32);
+        {
+            uint64_t mine = KEY_SENTINEL;
+            for (uint32_t l = tid; l < n_lists; l += nthr) {
+                const uint64_t v = __ldcg(keys + (size_t)l * k + k - 1);
+                mine = v < mine ? v : mine;
+            }
+            mine = ~warp_max_u64(~mine);
+            if (lane == 0 && mine != KEY_SENTINEL) atomicMin(&s_tT, (unsigned long long)mine);
+        }
+        if (k <= n_lists) {
+            for (uint32_t l = tid; l < n_lists; l += nthr) {
+                const uint64_t h = __ldcg(keys + (size_t)l * k);
+                cand[l] = h;
+                cg[l] = h != KEY_SENTINEL ? group_of(p, key_row(h)) : COLUMN_MISSING;
+            }
+            named_bar_sync(1, CW * 32);
+            group_firsts(cand, cg, cf, n_lists, tid, nthr, nullptr);
+            named_bar_sync(1, CW * 32);
+            for (uint32_t l = tid; l < n_lists; l += nthr)
+                if (cf[l] && group_rank(cand, cf, n_lists, cand[l]) == k - 1) atomicMin(&s_tT, (unsigned long long)cand[l]);
+        }
+        named_bar_sync(1, CW * 32);
+        const uint64_t T = s_tT;
+        for (uint32_t i = tid; i < n; i += nthr) {
+            const uint64_t key = __ldcg(keys + i);
+            if (key <= T && key != KEY_SENTINEL) {
+                const uint32_t e = atomicAdd(&s_tm, 1u);
+                cand[e] = key;
+                cg[e] = group_of(p, key_row(key));
+            }
+        }
+        named_bar_sync(1, CW * 32);
+        const uint32_t m = s_tm;
+        group_firsts(cand, cg, cf, m, tid, nthr, &s_tkept);
+        named_bar_sync(1, CW * 32);
+        for (uint32_t e = tid; e < m; e += nthr) {
+            if (!cf[e]) continue;
+            const uint32_t r = group_rank(cand, cf, m, cand[e]);
+            if (r < k) top[qi * k + r] = cand[e];
+        }
+        for (uint32_t r = s_tkept + tid; r < k; r += nthr) top[qi * k + r] = KEY_SENTINEL;
+        named_bar_sync(1, CW * 32);   // cand is reused by the next query; top is complete
+    }
+    for (uint32_t i = tid; i < p.nq_valid * k; i += nthr) {
+        const uint64_t key = top[i];
+        const bool valid = key != KEY_SENTINEL;
+        p.out_dists[i] = valid ? key_dist(key) : __int_as_float(0x7f800000);
+        p.out_rows[i] = valid ? (int64_t)(p.row_base + key_row(key)) : -1;
+        p.out_groups[i] = valid ? group_of(p, key_row(key)) : COLUMN_MISSING;
+    }
+    for (uint32_t qi = tid; qi < p.nq_valid; qi += nthr) {
+        int c = 0;
+        for (uint32_t j = 0; j < k; j++) c += top[qi * k + j] != KEY_SENTINEL;
+        p.out_counts[qi] = c;
+    }
+}
+
 // D += A B: A 16 x 32 int8 (row-major fragment a0..a3), B 32 x 8 int8 (b0, b1), int32 accumulators (exact)
 __device__ __forceinline__ void mma_m16n8k32_s8(int (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
     asm volatile("mma.sync.aligned.m16n8k32.row.col.s32.s8.s8.s32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
@@ -303,7 +527,7 @@ __device__ __forceinline__ void mma_m16n8k16_f16(float (&c)[4], uint32_t a0, uin
                  : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
 
-template <int METRIC, int NQ, int R, bool RANGE, bool INLINE, int HALF = 0, bool DEBUG = false>
+template <int METRIC, int NQ, int R, bool RANGE, bool INLINE, int HALF = 0, bool DEBUG = false, bool GROUP = false>
 __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) {
     constexpr int V = R * NQ;
     static_assert(V <= 32 && (V & (V - 1)) == 0, "R*NQ must be a power of two <= 32");
@@ -320,6 +544,8 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
     constexpr bool Q8 = HALF == 3;
     static_assert(!Q8 || !RANGE || DEBUG, "the int8 shadow takes single kNN queries");
     constexpr bool HMMA = HALF >= 2;   // tensor-core consumers: fp16 or int8
+    // GROUP (scan_kernel_grouped): k <= 32 replace-the-maximum lists of distinct groups (see group_list_insert)
+    static_assert(!GROUP || (!RANGE && !INLINE && !HALF), "grouped search is an fp32 kNN scan of prepared queries");
     extern __shared__ __align__(128) unsigned char smem[];
     // fallback launch behind a shadow scan: nothing to do when that one certified its answer
     if (NQ == 1 && p.run_if && *reinterpret_cast<const volatile uint32_t*>(p.run_if) == 0) return;   // (single queries only)
@@ -338,7 +564,7 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
     float4* ring = reinterpret_cast<float4*>(smem);
     float4* qs = ring + (size_t)S * p.stage_f4;                                   // [NQ][ld4]
     const uint32_t lcap = p.list_cap;             // slots per (warp, query) list
-    const bool buffered = lcap > k;               // append buffer + compaction instead of replace-max
+    const bool buffered = !GROUP && lcap > k;     // append buffer + compaction instead of replace-max
     // float4 per query in shared memory (HALF: ld4 counts 8-half units, Q8: 16-byte units)
     const uint32_t ldq4 = Q8 ? 4 * ld4 : (HALF ? 2 * ld4 : ld4);
     // HMMA: the query once more as halves of q * 2^t ([ld4] 16-byte units), behind the fp32 copy the re-rank reads;
@@ -348,6 +574,9 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
     uint64_t* full = lists + (RANGE ? 0 : (size_t)CW * NQ * lcap);                // [S]
     uint64_t* empty = full + S;                                                   // [S]
     StageMeta* meta = reinterpret_cast<StageMeta*>(empty + S);                    // [S]
+    // GROUP: fold scratch keys [64 + CW k] | the warp lists' groups [CW][NQ][k] | fold scratch groups, flags [64 + CW k] each
+    uint64_t* gscr = reinterpret_cast<uint64_t*>(meta + S);
+    int32_t* lgroups = reinterpret_cast<int32_t*>(gscr + (GROUP ? 64 + CW * k : 0));
 
     float half_qn = 0.f;                                                           // HALF: |q|^2
     float half_margin = 0.f;                                                       // HALF range mode: candidate margin
@@ -362,6 +591,8 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
     }
     if (!RANGE)
         for (uint32_t i = tid; i < (uint32_t)CW * NQ * lcap; i += blockDim.x) lists[i] = KEY_SENTINEL;
+    if constexpr (GROUP)
+        for (uint32_t i = tid; i < (uint32_t)CW * NQ * k; i += blockDim.x) lgroups[i] = COLUMN_MISSING;
     if (INLINE) {
         // the raw query comes with the launch: pad it to ld and, for cosine, normalise it with prep_queries_kernel's
         // exact arithmetic (lane l sums elements l, l+32, ... with fmaf, butterfly over the lanes, v * inv)
@@ -794,6 +1025,24 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
                     unsigned long long pos = atomicAdd(p.range_counts + my_q, 1ull);
                     if (pos < p.max_hits) p.range_keys[(size_t)my_q * p.max_hits + pos] = key;
                 }
+            } else if constexpr (GROUP) {
+                // the row's group is read only for rows that beat the threshold: the pass moves the bytes of a plain search
+                int32_t grp = COLUMN_MISSING;
+                if (ok && key < thr) grp = group_of(p, row);
+                unsigned m = __ballot_sync(0xffffffffu, ok && key < thr && grp != COLUMN_MISSING);   // no group: not a candidate
+                while (m) {
+                    const int src = __ffs(m) - 1;
+                    m &= m - 1;
+                    const uint64_t ckey = shfl_u64(key, src);
+                    const uint64_t cthr = shfl_u64(thr, src);
+                    const int cq = __shfl_sync(0xffffffffu, my_q, src);
+                    const int32_t cg = __shfl_sync(0xffffffffu, grp, src);
+                    if (ckey < cthr) {
+                        const size_t li = ((size_t)warp * NQ + cq) * k;
+                        const uint64_t nthr = group_list_insert(lists + li, lgroups + li, k, ckey, cg, cthr, lane);
+                        if (my_q == cq) thr = nthr;
+                    }
+                }
             } else {
                 unsigned m = __ballot_sync(0xffffffffu, ok && key < thr);
                 if (!buffered) {
@@ -842,7 +1091,22 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
     }
     if (p.timeline && tid == 0) p.timeline[blockIdx.x * 16 + 2] = global_timer_ns();
     const uint32_t nthr = (uint32_t)CW * 32u;  // consumer threads (the producer warps have left)
-    if (!RANGE) {
+    if constexpr (GROUP) {
+        // every list of this warp ascending with its groups, then the block's k best groups per query
+        __syncwarp();
+        for (uint32_t qi = 0; qi < (uint32_t)NQ && qi < p.nq_valid; qi++) {
+            const size_t li = ((size_t)warp * NQ + qi) * k;
+            uint64_t v = (uint32_t)lane < k ? lists[li + lane] : KEY_SENTINEL;
+            int32_t g = (uint32_t)lane < k ? lgroups[li + lane] : COLUMN_MISSING;
+            warp_bitonic_sort_kg(v, g, lane);
+            if ((uint32_t)lane < k) {
+                lists[li + lane] = v;
+                lgroups[li + lane] = g;
+            }
+        }
+        named_bar_sync(1, CW * 32);
+        group_fold<NQ>(p, lists, lgroups, gscr, lgroups + (size_t)CW * NQ * k, CW, (uint32_t)tid, nthr);
+    } else if (!RANGE) {
         // --------------------------------------------- fold the CW warp lists into one per query
         if (buffered) {
             // last compaction: every list of this warp ascending, k slots valid-or-sentinel
@@ -950,7 +1214,9 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
     if (s_ticket != gridDim.x - 1) return;
     __threadfence();
     if (p.timeline && tid == 0) p.timeline[blockIdx.x * 16 + 10] = global_timer_ns();       // last CTA: past the fence
-    if (!RANGE && p.fused) {
+    if constexpr (GROUP) {
+        group_tail<NQ>(p, smem, CW, (uint32_t)tid, nthr, lane);
+    } else if (!RANGE && p.fused) {
         // The ring is idle now: reuse it.  cand[fused_cap] | top[nq_valid][k]
         uint64_t* cand = reinterpret_cast<uint64_t*>(ring);
         uint64_t* top = cand + p.fused_cap;
@@ -1203,6 +1469,11 @@ __device__ __forceinline__ void scan_body(const ScanParams& p, const float* iq) 
 template <int METRIC, int NQ, int R, bool RANGE>
 __global__ void __launch_bounds__(scan_max_threads<NQ>(), 1) scan_kernel(const ScanParams p) {
     scan_body<METRIC, NQ, R, RANGE, false>(p, nullptr);
+}
+// grouped search (mlv_index_search_grouped): the k nearest groups of ScanParams::group_col, one best row each; fused tail only
+template <int METRIC, int NQ, int R>
+__global__ void __launch_bounds__(scan_max_threads<NQ>(), 1) scan_kernel_grouped(const ScanParams p) {
+    scan_body<METRIC, NQ, R, false, false, 0, false, true>(p, nullptr);
 }
 // one query over the fp16 shadow of the rows, exact re-rank + certificate in the fused tail (ScanParams::rows_exact)
 template <int METRIC, int R, bool RANGE = false>

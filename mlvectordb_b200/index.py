@@ -20,7 +20,7 @@ Deliberate differences:
     ``rebuild_threshold`` is compacted on the device and ``is_rebuild_required`` stays False, so
     ``QueryProcessor.delete`` never takes the reference's rebuild path that wipes the *other*
     namespaces (Q6).  ``auto_compact=False`` restores the reference's flag behaviour.
-Additive (no reference code; README-only intent): ``search_batch``, ``filter=``,
+Additive (no reference code; README-only intent): ``search_batch``, ``filter=``, ``group_by=``,
 ``range_search``, ``dimension``, ``add_matrix``, ``info``.
 """
 from __future__ import annotations
@@ -247,6 +247,19 @@ class GpuIndex:
             ns.where_cache[key] = prepared
         return prepared
 
+    @staticmethod
+    def _group_column(ns: _Namespace, group_by: str) -> Optional[int]:
+        """Device column of metadata key ``group_by``, or None when no row ever had the key (no groups at all).  A key
+        kept on the host only cannot be grouped on the device, and there is no host grouping."""
+        if ns.codec.kind(group_by) == "host":
+            raise NotDeviceEvaluable(f"metadata key {group_by!r} is not held as a device column; it cannot be grouped by")
+        return ns.codec.column_index(group_by)
+
+    @staticmethod
+    def _check_group_k(top_k: int) -> None:
+        if int(top_k) > _capi.MAX_GROUP_K:
+            raise ValueError(f"group_by supports top_k <= {_capi.MAX_GROUP_K}, got {top_k}")
+
     # ------------------------------------------------------------------ IndexProtocol
     def add(self, vectors: Iterable[VectorProtocol], namespace: str) -> None:
         """reference index.py:50-67"""
@@ -285,8 +298,14 @@ class GpuIndex:
         self._maybe_compact(ns)
 
     def search(self, query: VectorDTO, top_k: int, namespace: str, metric: str,
-               filter: FilterArg = None) -> List[SearchResult]:
-        """reference index.py:91-129 (``filter`` is additive)."""
+               filter: FilterArg = None, group_by: Optional[str] = None) -> List[SearchResult]:
+        """reference index.py:91-129 (``filter`` and ``group_by`` are additive).
+
+        ``group_by``: a metadata key; the result is then the ``top_k`` (<= 32) nearest *groups* -- rows with equal
+        values of the key (Python equality) -- each reported by its nearest row, nearest group first.  Rows without the
+        key belong to no group (``mlv_index_search_grouped``)."""
+        if group_by is not None:
+            self._check_group_k(top_k)
         ns = self._ns.get(namespace)
         if ns is None:
             return []
@@ -299,7 +318,13 @@ class GpuIndex:
         q = np.asarray(query.values, dtype=np.float32).reshape(-1)
         if q.shape[0] != ns.dim:
             return []  # the reference swallows hnswlib's dimension RuntimeError into [] (index.py:110-119)
-        dists, rows, counts = ns.shard.search(q[None, :], top_k, self._filter_mask(ns, filter))
+        if group_by is None:
+            dists, rows, counts = ns.shard.search(q[None, :], top_k, self._filter_mask(ns, filter))
+        else:
+            column = self._group_column(ns, group_by)
+            if column is None:
+                return []
+            dists, rows, _, counts = ns.shard.search_grouped(q[None, :], top_k, column, self._filter_mask(ns, filter))
         c = int(counts[0])
         raw = ns.ids[rows[0, :c]].tobytes()          # the hits' uuid bytes in one gather (label -> UUID, reference index.py:123)
         scores = dists[0, :c].tolist()
@@ -417,11 +442,14 @@ class GpuIndex:
         ns.touch()
 
     def search_batch(self, queries: np.ndarray, top_k: int, namespace: str, metric: Optional[str] = None,
-                     filter: FilterArg = None):
+                     filter: FilterArg = None, group_by: Optional[str] = None):
         """Batched search -> (rows i64 [nq,k] (-1 padded), scores f32 [nq,k], counts i32 [nq]).
 
-        Scores follow ``search``: hnswlib-form distances, ``1 - d`` when ``metric == "cosine"``.
+        Scores follow ``search``: hnswlib-form distances, ``1 - d`` when ``metric == "cosine"``.  ``group_by`` as in
+        ``search``: row i of the result holds query i's nearest groups, one row each.
         """
+        if group_by is not None:
+            self._check_group_k(top_k)
         q = np.ascontiguousarray(queries, dtype=np.float32)
         if q.ndim == 1:
             q = q[None, :]
@@ -431,7 +459,13 @@ class GpuIndex:
         k = min(int(top_k), active)
         if ns is None or k < 1 or q.shape[1] != ns.dim:
             return (np.full((nq, 0), -1, np.int64), np.empty((nq, 0), np.float32), np.zeros(nq, np.int32))
-        dists, rows, counts = ns.shard.search(q, k, self._filter_mask(ns, filter))
+        if group_by is None:
+            dists, rows, counts = ns.shard.search(q, k, self._filter_mask(ns, filter))
+        else:
+            column = self._group_column(ns, group_by)
+            if column is None:
+                return (np.full((nq, 0), -1, np.int64), np.empty((nq, 0), np.float32), np.zeros(nq, np.int32))
+            dists, rows, _, counts = ns.shard.search_grouped(q, k, column, self._filter_mask(ns, filter))
         if (metric if metric is not None else self._space) == "cosine":
             dists = (1.0 - dists.astype(np.float64)).astype(np.float32)
         return rows, dists, counts

@@ -88,10 +88,13 @@ class GpuQueryProcessor:
         self._touch(namespace)
 
     def find_similar(self, query: VectorDTO, top_k: int, namespace: str = "default", metric: str = "cosine",
-                     filter: MetadataFilter = None, enrich: bool = True) -> List[dict]:  # noqa: A002
-        """reference query_processor.py:26-49; ``filter`` / ``enrich`` are additive."""
+                     filter: MetadataFilter = None, enrich: bool = True,  # noqa: A002
+                     group_by: Optional[str] = None) -> List[dict]:
+        """reference query_processor.py:26-49; ``filter`` / ``enrich`` / ``group_by`` are additive.  ``group_by``: the
+        ``top_k`` (<= 32) nearest groups of that metadata key, each as its nearest vector (``GpuIndex.search``)."""
+        grouped = {"group_by": group_by} if group_by is not None else {}
         results = self._index.search(query, top_k=top_k, namespace=namespace, metric=metric,
-                                     filter=self._resolve_filter(namespace, filter))
+                                     filter=self._resolve_filter(namespace, filter), **grouped)
         if not results:
             return []
         return self._enrich([(r.vector_id, r.score) for r in results], namespace, enrich)
@@ -122,13 +125,14 @@ class GpuQueryProcessor:
     # ------------------------------------------------------------------ additive surface
     def find_similar_batch(self, queries: Sequence[Union[VectorDTO, Sequence[float]]], top_k: int,
                            namespace: str = "default", metric: str = "cosine", filter: MetadataFilter = None,  # noqa: A002
-                           enrich: bool = True) -> List[List[dict]]:
+                           enrich: bool = True, group_by: Optional[str] = None) -> List[List[dict]]:
         """One result list per query, each exactly what ``find_similar`` returns for that query."""
         q = np.asarray([getattr(v, "values", v) for v in queries], dtype=np.float32)
         if q.ndim != 2 or q.shape[0] == 0:
             return [[] for _ in range(len(queries))]
+        grouped = {"group_by": group_by} if group_by is not None else {}
         rows, scores, counts = self._index.search_batch(q, top_k, namespace, metric=metric,
-                                                        filter=self._resolve_filter(namespace, filter))
+                                                        filter=self._resolve_filter(namespace, filter), **grouped)
         out = []
         for i in range(q.shape[0]):
             n = int(counts[i])

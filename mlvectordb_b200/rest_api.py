@@ -14,6 +14,9 @@ What the GPU index can do beyond the reference becomes reachable from the produc
   ``radius`` (range search instead of top-k) and ``include_values`` (``false`` skips the k x d float payload
   that dominates a response at GPU speeds -- rank 2);
 * ``POST /search/batch``: many queries per request (tensor-core path from 5 queries on a >= 1 GB matrix);
+* ``group_by`` (a metadata key) on ``POST /search``, ``POST /search/batch``, ``POST /query/knn`` and ``POST /query/hybrid``:
+  the ``top_k`` (<= 32) nearest groups of rows sharing the key's value, each reported by its nearest row.  Combined with
+  ``radius``, with ``top_k`` > 32 or with a key the index keeps on the host only, the request gets 400;
 * the routes the reference only documents (``README.md:325-333``) with the request shapes of its example
   client (``examples/api_client.py:26-74``): ``POST /query/knn`` (``vector``, ``k``), ``POST /query/range``
   (``vector``, ``radius``), ``POST /query/similarity`` (``vector``, ``threshold``, ``metric``: cosine
@@ -36,7 +39,8 @@ from uuid import UUID
 from fastapi import FastAPI, HTTPException, Query, Request, Response, status
 from pydantic import BaseModel, Field
 
-from ._capi import format_f32_json
+from ._capi import MAX_GROUP_K, format_f32_json
+from .index import NotDeviceEvaluable
 from .interfaces import VectorDTO
 
 
@@ -54,6 +58,7 @@ class VectorSearchRequest(BaseModel):
     filter: Optional[Dict[str, Any]] = None
     radius: Optional[float] = None
     include_values: bool = True
+    group_by: Optional[str] = None
 
 
 class VectorSearchResult(BaseModel):
@@ -84,6 +89,7 @@ class BatchSearchRequest(BaseModel):
     metric: str = "cosine"
     filter: Optional[Dict[str, Any]] = None
     include_values: bool = False
+    group_by: Optional[str] = None
 
 
 class QueryRequest(BaseModel):
@@ -97,6 +103,7 @@ class QueryRequest(BaseModel):
     namespace: str = "default"
     include_values: bool = True
     type: Optional[str] = None
+    group_by: Optional[str] = None
 
 
 def _constraints(raw: Optional[Dict[str, Any]]) -> Optional[Dict[str, Any]]:
@@ -127,6 +134,16 @@ def _encode_hits(hits) -> bytes:
             json.dumps(metadata, default=str).encode() if metadata else b"{}",
             repr(score).encode() if math.isfinite(score) else json.dumps(score).encode()))
     return b"[" + b",".join(parts) + b"]"
+
+
+def _check_group_by(group_by: Optional[str], radius: Optional[float], top_k: int) -> None:
+    """400 for the ``group_by`` requests the index cannot answer."""
+    if group_by is None:
+        return
+    if radius is not None:
+        raise HTTPException(status_code=status.HTTP_400_BAD_REQUEST, detail="group_by cannot be combined with radius")
+    if top_k > MAX_GROUP_K:
+        raise HTTPException(status_code=status.HTTP_400_BAD_REQUEST, detail=f"group_by supports top_k <= {MAX_GROUP_K}")
 
 
 def _json(payload: bytes) -> Response:
@@ -163,7 +180,8 @@ class GpuRestAPI:
         self.logger.error("%s: %s", what, exc, exc_info=True)
         raise HTTPException(status_code=status.HTTP_500_INTERNAL_SERVER_ERROR, detail=f"{what}: {exc}")
 
-    def _search(self, query: List[float], top_k: int, namespace: str, metric: str, flt, radius, include_values: bool):
+    def _search(self, query: List[float], top_k: int, namespace: str, metric: str, flt, radius, include_values: bool,
+                group_by: Optional[str] = None):
         qp = self.query_processor
         dto = VectorDTO(values=query, metadata={})
         extra = {}
@@ -171,11 +189,19 @@ class GpuRestAPI:
             extra["filter"] = flt
         if not include_values:
             extra["enrich"] = False
+        if group_by is not None:
+            extra["group_by"] = group_by
         if radius is not None:
             return qp.find_in_range(dto, radius, namespace=namespace, metric=metric, **extra)
         # without additive fields this is exactly the reference's call (rest_api.py:178-183), so any
         # QueryProcessorProtocol implementation works behind the reference routes
         return qp.find_similar(query=dto, top_k=top_k, namespace=namespace, metric=metric, **extra)
+
+    def _bad_group_by(self, group_by: Optional[str], what: str, exc: Exception):
+        """A grouped request over a key the device cannot group by is the client's error (400); anything else is not."""
+        if group_by is None:
+            self._fail(what, exc)
+        raise HTTPException(status_code=status.HTTP_400_BAD_REQUEST, detail=str(exc))
 
     # ------------------------------------------------------------------ routes
     def _setup_routes(self):
@@ -200,19 +226,26 @@ class GpuRestAPI:
 
         @app.post("/search", response_model=List[VectorSearchResult])
         async def search_similar(search_request: VectorSearchRequest, namespace: str = Query("default")):
+            r = search_request
+            _check_group_by(r.group_by, r.radius, r.top_k)
             try:
-                r = search_request
                 return _json(_encode_hits(self._search(r.query, r.top_k, namespace, r.metric, _constraints(r.filter), r.radius,
-                                                       r.include_values)))
+                                                       r.include_values, r.group_by)))
+            except NotDeviceEvaluable as e:
+                self._bad_group_by(r.group_by, "Search failed", e)
             except Exception as e:  # noqa: BLE001
                 self._fail("Search failed", e)
 
         @app.post("/search/batch", response_model=List[List[VectorSearchResult]])
         async def search_batch(batch: BatchSearchRequest, namespace: str = Query("default")):
+            _check_group_by(batch.group_by, None, batch.top_k)
+            grouped = {"group_by": batch.group_by} if batch.group_by is not None else {}
             try:
                 per_query = qp.find_similar_batch(batch.queries, batch.top_k, namespace=namespace, metric=batch.metric,
-                                                  filter=_constraints(batch.filter), enrich=batch.include_values)
+                                                  filter=_constraints(batch.filter), enrich=batch.include_values, **grouped)
                 return _json(b"[" + b",".join(_encode_hits(hits) for hits in per_query) + b"]")
+            except NotDeviceEvaluable as e:
+                self._bad_group_by(batch.group_by, "Batch search failed", e)
             except Exception as e:  # noqa: BLE001
                 self._fail("Batch search failed", e)
 
@@ -275,11 +308,14 @@ class GpuRestAPI:
                         radius = None
                     if kind == "hybrid" and not req.filter:
                         raise HTTPException(status_code=status.HTTP_400_BAD_REQUEST, detail="filter is required")
+                    _check_group_by(req.group_by, radius, req.k)
                     hits = self._search(req.vector, req.k, req.namespace, req.metric, _constraints(req.filter), radius,
-                                        req.include_values)
+                                        req.include_values, req.group_by)
                     return _json(b'{"type":"%s","count":%d,"results":%s}' % (kind.encode(), len(hits), _encode_hits(hits)))
                 except HTTPException:
                     raise
+                except NotDeviceEvaluable as e:
+                    self._bad_group_by(req.group_by, f"{kind} query failed", e)
                 except Exception as e:  # noqa: BLE001
                     self._fail(f"{kind} query failed", e)
             handler.__name__ = f"query_{kind}"

@@ -180,6 +180,27 @@ class DeviceShard:
                                                 dists.ctypes.data, rows.ctypes.data, counts.ctypes.data))
         return dists, rows, counts
 
+    def search_grouped(self, queries: np.ndarray, k: int, column: int, filt=None):
+        """Grouped search (``mlv_index_search_grouped``): the k nearest groups of device column ``column``, one best row
+        per group.  -> (dists f32 [nq,k] ascending, rows i64 [nq,k], groups i32 [nq,k] (``COLUMN_MISSING`` padded),
+        counts i32 [nq]); 1 <= k <= ``_capi.MAX_GROUP_K``."""
+        q = np.ascontiguousarray(queries, dtype=np.float32)
+        if q.ndim == 1:
+            q = q[None, :]
+        if q.ndim != 2 or q.shape[1] != self.dim:
+            raise ValueError(f"expected queries of dimension {self.dim}, got shape {q.shape}")
+        nq = q.shape[0]
+        dists = np.empty((nq, k), dtype=np.float32)
+        rows = np.empty((nq, k), dtype=np.int64)
+        groups = np.empty((nq, k), dtype=np.int32)
+        counts = np.empty(nq, dtype=np.int32)
+        fw = self._filter_words(filt)
+        with _bound(self, filt):
+            self._ck(self._lib.mlv_index_search_grouped(self._h, q.ctypes.data, nq, int(k), int(column),
+                                                        fw.ctypes.data if fw is not None else None, dists.ctypes.data,
+                                                        rows.ctypes.data, groups.ctypes.data, counts.ctypes.data))
+        return dists, rows, groups, counts
+
     def search_device(self, q_ptr: int, nq: int, k: int, out_d_ptr: int, out_r_ptr: int, out_c_ptr: int,
                       filter_ptr: int = 0, stream: int = 0) -> None:
         """All pointers are device addresses (e.g. ``tensor.data_ptr()``); enqueues on ``stream``
