@@ -1059,7 +1059,7 @@ int mlv_index_range_search_device(mlv_index_t h, const float* queries_dev, uint3
     r.p.radius = radius;
     r.p.max_hits = max_hits;
     for (uint32_t q = 0; q < nq; q++) CK(h, launch_range(h, r, q, st));
-    CK(h, cudaFuncSetAttribute(range_finish_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(SELECT_MAX_P * 8)));
+    CK(h, raise_smem_once<range_finish_kernel>(SELECT_MAX_P * 8));
     range_finish_kernel<<<nq, SELECT_THREADS, (size_t)SELECT_MAX_P * 8, st>>>(r.d_keys, r.d_counts, r.slots, max_hits, h->row_base,
                                                                             out_dists_dev, out_rows_dev, (unsigned long long*)out_counts_dev);
     h->launches++;
@@ -1129,7 +1129,7 @@ int mlv_index_range_search_exchange_device(mlv_index_t h, const float* queries_d
     const uint64_t share = XCHG_SLOT_KEYS / x.world;
     int rc;
     if (h->rows == h->n_deleted) {   // nothing to scan here, but the peers wait for this rank's (empty) list
-        CK(h, cudaFuncSetAttribute(range_exchange_only_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)(XCHG_SLOT_KEYS * 8)));
+        CK(h, raise_smem_once<range_exchange_only_kernel>(XCHG_SLOT_KEYS * 8));
         for (uint32_t q = 0; q < nq; q++) {
             x.seq = ++h->xseq;
             range_exchange_only_kernel<<<1, 256, (size_t)XCHG_SLOT_KEYS * 8, st>>>(x, out_dists_dev + (size_t)q * XCHG_SLOT_KEYS,
@@ -1250,7 +1250,7 @@ int mlv_merge_topk(int device, const float* dists_dev, const int64_t* rows_dev, 
     if ((uint64_t)n_lists * k > SELECT_MAX_P) return MLV_E_UNSUPPORTED;
     DeviceGuard g(device);
     if (!g.ok) return MLV_E_CUDA;
-    if (ensure_select_attrs(device) != cudaSuccess) return MLV_E_CUDA;
+    if (raise_smem_once<merge_pairs_kernel>(SELECT_MAX_P * 8) != cudaSuccess) return MLV_E_CUDA;
     MergePairsParams p{};
     p.dists = dists_dev;
     p.rows = rows_dev;
@@ -1338,7 +1338,8 @@ int mlv_index_debug_gemm(mlv_index_t h, const float* queries, uint32_t nq, float
     // one round over every row tile at threshold +inf: each live row is a candidate of every query
     const uint32_t tiles = (uint32_t)((h->rows + GEMM_BM - 1) / GEMM_BM);
     mlv_gemm_rounds_cfg_t c{};
-    c.passes = h->tune_gemm_passes == 1 ? 1u : (h->tune_gemm_passes == GEMM_TIER_F16 ? (uint32_t)GEMM_TIER_F16 : 3u);   // which tier's distances
+    const GemmTierRule tiers = gemm_tier_rule(h, 1);   // the distances of the last tier a batch runs before the scan
+    c.passes = tiers.one_pass && !tiers.second ? (tiers.half ? (uint32_t)GEMM_TIER_F16 : 1u) : 3u;
     c.bn = gemm_tile_width(h, nq);
     c.cap = pow2_ceil((uint32_t)h->rows);
     c.n_rounds = 1;

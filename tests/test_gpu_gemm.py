@@ -481,3 +481,56 @@ def test_cta_pair_kernel_equals_the_single_tile_kernel(space):
     if space != "cosine":
         assert ref[1][7, 0] == n - 1 or not live[n - 1]
     s.close()
+
+
+@pytest.mark.parametrize("wide", [0, None])
+@pytest.mark.parametrize("passes", [0, 1, 2, 3])
+def test_each_round_is_one_timed_region_and_two_launches(passes, wide):
+    """With timing on, a batch adds one timed region per GEMM round.  Once the row norms and the fp16 shadow exist, it
+    launches the query preparation, then per tier the query split, a GEMM and a refine per round and the re-rank, and the
+    gather / scatter around a 3xTF32 tier that re-runs failing queries.  wide None = the default (CTA pairs)."""
+    n, dim, nq, k = 20_000, 128, 300, 10       # 300 queries: 256-wide tiles, the CTA-pair kernel on one-pass tiers
+    rng = np.random.default_rng(31)
+    s = _shard(dim, "l2")
+    s.add(rng.standard_normal((n, dim), dtype=np.float32))
+    Q = rng.standard_normal((nq, dim), dtype=np.float32)
+    s.set_tuning("gemm", 1)
+    s.set_tuning("gemm_passes", passes)
+    if wide is not None:
+        s.set_tuning("gemm_wide", wide)
+    s.set_timing(True)
+    s.search(Q, k)                             # builds the row norms and (passes 0, 2) the fp16 shadow
+    before, launches = s.gemm_stats(), s.kernel_launches()
+    s.search(Q, k)
+    after, launches = s.gemm_stats(), s.kernel_launches() - launches
+    d = {f: after[f] - before[f] for f in ("searches", "rounds", "fast_queries", "half_queries", "fallback_queries")}
+    assert d["searches"] == 1 and d["rounds"] > 0 and d["fallback_queries"] == 0, d
+    assert d["half_queries"] == (d["fast_queries"] if passes in (0, 2) else 0), d
+    assert passes != 3 or d["fast_queries"] == 0, d
+    assert after["gemm_launches_timed"] == d["rounds"], (after["gemm_launches_timed"], d)   # gemm_stats drains the regions it reports
+    second = passes == 0 and d["fast_queries"] < nq
+    tiers = 2 if second else 1
+    assert launches == 1 + 2 * tiers + 2 * d["rounds"] + (2 if second else 0), (launches, d)
+    s.close()
+
+
+def test_debug_rounds_are_neither_counted_nor_timed():
+    """debug_gemm_rounds launches the query preparation, the split and a GEMM and a refine per round, and leaves the
+    search counters and the timed regions alone."""
+    n, dim, nq = 20_000, 128, 64
+    rng = np.random.default_rng(32)
+    s = _shard(dim, "l2")
+    s.add(rng.standard_normal((n, dim), dtype=np.float32))
+    Q = rng.standard_normal((nq, dim), dtype=np.float32)
+    s.set_timing(True)
+    s.set_tuning("gemm", 1)
+    s.search(Q, 10)                            # builds the row norms
+    before, launches = s.gemm_stats(), s.kernel_launches()
+    rounds = [(8, 96), (40, 96), (-(-n // 128), 96)]
+    for bn, passes in ((64, 1), (64, 3), (0, 2)):
+        s.debug_gemm_rounds(Q, passes=passes, bn=bn, cap=1024, rounds=rounds, kprime=96)
+    after, launches = s.gemm_stats(), s.kernel_launches() - launches
+    assert after["rounds"] == before["rounds"] and after["searches"] == before["searches"]
+    assert after["gemm_launches_timed"] == 0
+    assert launches == 3 * (2 + 2 * len(rounds)), launches
+    s.close()
